@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 3 --warmup 3
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
     python bench.py --impl reference ...          # the reference's own classes (oracle/_ref) on the host cores
+    python bench.py ... --dump-outputs DIR        # also write the last timed step's per-rollout metrics as DIR/*.npy
 
 Workload (config.workload): BASELINE.json configs[2] -- 10^5 lab_course rollouts per GPU with Monte-Carlo PID gains and
 mass/inertia perturbations, velocity 3.0 (config.ini) => 10 760 ticks each, 1.076e9 drone-sim-steps per GPU and step.  One "step" =
@@ -50,6 +51,7 @@ VELOCITY = 3.0               # config.ini:7
 FREQUENCY = 10               # config.ini:2
 TICKS_PER_ROLLOUT = 10_760   # lab_course at v = 3: 1076 table rows x 10 (read back from the plan in the GPU arm)
 METRIC = "drone-sim-steps/s"
+DUMP_BYTES = 64 << 20        # --dump-outputs budget over all files
 
 
 def parse():
@@ -62,7 +64,14 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the side measurements (other configs, K1 / K3 / RRT*, log mode, parity)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="wall-clock budget of the CPU baseline sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed paths returned in their last timed step as DIR/<name>.npy "
+                    f"(at most {DUMP_BYTES >> 20} MB in all: a fixed, seeded sample of rows when larger)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200: the reference arm reports rates only")
+    return args
 
 
 def workload_name(rollouts):
@@ -465,9 +474,13 @@ def run_b200(args):
     W = max(args.warmup, 3)
     sampler = ClockSampler(local) if rank == 0 else None
     ms_dev, clocks = timed(step_device, args.steps, W, sampler, after=drain)
+    dumped = {"metrics": gather.result(state["k"] - 1).cpu().numpy()} if args.dump_outputs and rank == 0 else None    # [total, 8] fp32
     n_ticks = state["n"]
     ms_e2e, _ = timed(step_e2e, args.steps, 2, wall=True)
     torch.cuda.synchronize()
+    if dumped is not None:
+        dumped["e2e_metrics"] = metrics_host.numpy()                                         # this rank's [B, 8] fp32
+        dump_outputs(args.dump_outputs, dumped)
     sim_steps = float(total) * n_ticks                                                       # whole job, one step
     value = sim_steps * args.steps / (ms_dev * 1e-3)
     e2e = sim_steps * args.steps / (ms_e2e * 1e-3)
@@ -700,6 +713,19 @@ def solve_rate(kernels, host_api, dev, flush, peaks):
                       "call": "uavb_minsnap_solve_f64_host (C ABI, pinned host buffers, chunked H2D -> K1 -> D2H pipeline, synchronous)",
                       "link_GBps": (h2d + d2h) / te / 1e9, "note": "bound by the host link: 932 B cross PCIe per solve, 804 of them device-to-host"}
     return out
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: every array as out_dir/<name>.npy.  An array larger than its share of DUMP_BYTES is cut to a fixed, seeded,
+    sorted sample of its rows, the same for every run with the same arguments, so two builds can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 4096                                                # room for the .npy header
+    for name, a in arrays.items():
+        if a.nbytes > share:
+            keep = share // (a.nbytes // len(a))
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def emit(line: dict) -> None:

@@ -257,20 +257,21 @@ def closed_loops():
     table = _generate_mission_trajectory(WAYPOINTS, OBSTACLES, 3.0, 0.01)
     rng = np.random.default_rng(99)
     var = {}
+    unused = ("fine", "cmd")                      # no test reads them for the variants; left out to keep the file under 1 MB
     res = fly(table, WAYPOINTS[0], lag=0, full_rate_ticks=0)
-    var.update({f"nolag_{k}": v for k, v in res.items() if k != "fine"})
+    var.update({f"nolag_{k}": v for k, v in res.items() if k not in unused})
     for j in range(3):
         gs, m, ins = rng.uniform(0.8, 1.2, 11), float(rng.uniform(0.9, 1.1)), rng.uniform(0.9, 1.1, 3)
         res = fly(table, WAYPOINTS[0], gain_scale=gs, mass_scale=m, inertia_scale=ins, full_rate_ticks=0)
-        var.update({f"mc{j}_{k}": v for k, v in res.items() if k != "fine"})
+        var.update({f"mc{j}_{k}": v for k, v in res.items() if k not in unused})
         var[f"mc{j}_gain_scale"], var[f"mc{j}_mass_scale"], var[f"mc{j}_inertia_scale"] = gs, np.array(m), ins
     wind = np.array([0.10, -0.06, 0.04])
     res = fly(table, WAYPOINTS[0], wind=wind, full_rate_ticks=0)
-    var.update({f"wind_{k}": v for k, v in res.items() if k != "fine"})
+    var.update({f"wind_{k}": v for k, v in res.items() if k not in unused})
     var["wind_force"] = wind
     blocker = np.vstack((OBSTACLES, [[8.0, 9.0, 3.0, 6.0, -4.0, -2.0]]))  # sits on the course: the flag must trip
     res = fly(table, WAYPOINTS[0], obstacles=blocker, full_rate_ticks=0)
-    var.update({f"hit_{k}": v for k, v in res.items() if k != "fine"})
+    var.update({f"hit_{k}": v for k, v in res.items() if k not in unused})
     var["hit_obstacles"] = blocker
     np.savez_compressed(os.path.join(HERE, "closed_loop_variants.npz"), **var)
     print("variants:", {k: float(v) for k, v in var.items() if k.endswith("final_dist") or k.endswith("first_collision_tick")})
@@ -358,7 +359,14 @@ def rrt():
     print("rrt.npz:", {k: v.shape for k, v in out.items() if k.startswith("path")}, "segment hits", int(hits.any(axis=1).sum()), "of", len(p))
 
 
+def scene():
+    """The reference's lab_course.xml, copied as is: tests/test_scene_reader.py checks the transcribed scene constants against it."""
+    import shutil
+    import uav_ac
+    shutil.copyfile(os.path.join(os.path.dirname(uav_ac.__file__), "simulation", "models", "lab_course.xml"), os.path.join(HERE, "lab_course.xml"))
+
+
 if __name__ == "__main__":
-    which = sys.argv[1:] or ["planning", "stages", "closed_loops", "actual_trajectory", "rrt"]
+    which = sys.argv[1:] or ["planning", "stages", "closed_loops", "actual_trajectory", "rrt", "scene"]
     for w in which:
         globals()[w]()

@@ -1,6 +1,6 @@
 """Scene reader without MuJoCo (SURVEY 8(f) rank 3): stdlib-XML extraction of what MujocoSimulation.__init__ reads
-(mujoco_sim.py:51-91, 258-347).  A small MJCF written here exercises the conversions and the error cases; when the
-reference checkout is present (build container only) its lab_course.xml must reproduce the transcribed constants."""
+(mujoco_sim.py:51-91, 258-347).  A small MJCF written here exercises the conversions and the error cases; the
+reference's own lab_course.xml, stored as tests/golden/lab_course.xml by make_golden.py, must reproduce the transcribed constants."""
 import os
 import textwrap
 
@@ -77,9 +77,9 @@ def test_reader_raises_like_the_reference(tmp_path, old, new, msg):
 
 
 def test_lab_course_xml_reproduces_the_transcribed_constants():
-    path = "/root/reference/uav_ac/simulation/models/lab_course.xml"
+    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "lab_course.xml")
     if not os.path.exists(path):
-        pytest.skip("reference checkout not present (GPU box): the transcribed constants are pinned in the build container")
+        pytest.skip("tests/golden/lab_course.xml not stored: run tests/golden/make_golden.py with the reference present")
     s = scene.load_scene(path)
     np.testing.assert_allclose(s.mission_waypoints, scene.LAB_COURSE_WAYPOINTS, rtol=0, atol=1e-15)
     np.testing.assert_allclose(s.obstacles, scene.LAB_COURSE_OBSTACLES, rtol=0, atol=1e-12)
