@@ -307,8 +307,40 @@ int uavb_rollout_targets_f64(const double* seg_coeffs, const int* seg_rows, cons
  * (minimum_snap.py:97-124) evaluated on the fly. */
 int uavb_rollout_f32(const uavb_rollout_args* args, void* stream);
 
-/* Same rollout with every state variable and operation in fp64 (validation of the fp32 path). */
+/* Same rollout with every state variable and operation in fp64 (validation of the fp32 path).  Waypoint missions only: caller
+ * tables (uavb_rollout_tables_f32) have no fp64 form. */
 int uavb_rollout_f64(const uavb_rollout_args* args, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * Caller-supplied trajectory tables: the seam TrajectoryController(controller, quad, trajectory, frequency) (main.py:10-61)
+ * flies ANY (N, 11) table [x y z vx vy vz ax ay az yaw spline_id], one row per outer period, the index clamped at the last row.
+ *
+ * uavb_table_targets_f64: tables [n_rows][11] fp64 (several tables may be packed one after the other) -> targets_out [n_rows]
+ * records of UAVB_TARGET_ROW_BYTES: x y z copied, velocity / acceleration rounded once to fp32, the yaw column (the set-point the
+ * reference feeds to yaw_controller, main.py:58) as the heading direction (cos yaw, sin yaw) computed in fp64 -- yaw and
+ * yaw + 2 pi k are the same set-point, as in controller.py:156-168.  No hold-last-valid rule is applied (that belongs to table
+ * generation, minimum_snap.py:126-136); the spline_id column is ignored; non-finite values pass through (the rollout then reports
+ * UAVB_ROLLOUT_NONFINITE). */
+int uavb_table_targets_f64(const double* tables, long long n_rows, void* targets_out, void* stream);
+
+typedef struct uavb_table_set {
+  const void*      rows;         /* DEVICE [n_rows] UAVB_TARGET_ROW_BYTES records (uavb_table_targets_f64)                          */
+  const long long* offsets;      /* DEVICE [n_tables + 1]: table t = rows [offsets[t], offsets[t+1]), >= 1 row each                  */
+  const int*       table_index;  /* DEVICE [B] table of every rollout, 0 <= table_index[b] < n_tables; NULL = rollout b flies table b
+                                    (n_tables == B)                                                                                    */
+  int              n_tables;
+  int              shared_rows;  /* > 0: ONE table of this many rows flown by every rollout (offsets / table_index NULL, n_tables unused) */
+} uavb_table_set;
+
+/* The fp32 rollout of uavb_rollout_f32 with the set-points read from caller tables: inner_per_outer ticks per table row, the row
+ * index clamped at each rollout's own last row (main.py:61).  Every mission-segment field of `args` must be NULL / 0 (seg_*,
+ * mission_seg_*, n_seg_shared, shared_targets, n_target_rows), otherwise UAVB_EINVAL; dt_outer is not read (the controller's outer
+ * period is veh.dt * inner_per_outer).  Everything else keeps its meaning: Monte-Carlo overrides, obstacle sets, floor, state log,
+ * flown-path list, start / goal strides, n_slices, carry / resume (the carry holds the row relative to the rollout's table: resume
+ * with the same table set) and index_base.  A shared table runs the shared-mission kernels of uavb_rollout_f32; per-rollout tables
+ * run kernels that read one record per lane and outer period.  The table set is not range-checked on the device: offsets must be
+ * non-decreasing with >= 1 row per table and table_index inside [0, n_tables). */
+int uavb_rollout_tables_f32(const uavb_rollout_args* args, const uavb_table_set* tables, void* stream);
 
 /* Fill `veh` with the lab_course.xml vehicle and the gains of Quad.__init__ (quad.py:54-73). */
 void uavb_vehicle_defaults(uavb_vehicle* veh);

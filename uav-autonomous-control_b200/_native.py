@@ -36,6 +36,7 @@ SYMBOLS = (
     "uavb_minsnap_table_hits_f64", "uavb_minsnap_correct_f64", "uavb_minsnap_pack_f64", "uavb_plan_shared_f64", "uavb_minsnap_constraints_f64",
     "uavb_rollout_targets_f64", "uavb_rollout_f32", "uavb_rollout_f64", "uavb_vehicle_defaults", "uavb_stage_f32", "uavb_mc_uniform_f32",
     "uavb_mc_missions_f64", "uavb_measure_fma_peak", "uavb_measure_fma_rates", "uavb_minsnap_solve_f64_host", "uavb_fly_mission_host", "uavb_rrt_workspace_bytes", "uavb_rrt_star_f64", "uavb_segments_hit_aabbs_f64",
+    "uavb_table_targets_f64", "uavb_rollout_tables_f32",
 )
 
 
@@ -70,6 +71,11 @@ class RolloutArgs(Structure):
         ("traj_out", c_void_p), ("traj_count_out", c_void_p), ("traj_max_samples", c_int), ("traj_gate_z", c_double), ("traj_interval", c_double),
         ("ground_on", c_int), ("ground_z", c_double), ("pair_kernel_only", c_int), ("log_tma", c_int),
     ]
+
+
+class TableSet(Structure):
+    """struct uavb_table_set (include/uavb.h): caller trajectory tables for uavb_rollout_tables_f32."""
+    _fields_ = [("rows", c_void_p), ("offsets", c_void_p), ("table_index", c_void_p), ("n_tables", c_int), ("shared_rows", c_int)]
 
 
 class StageArgs(Structure):
@@ -126,6 +132,8 @@ def lib() -> ctypes.CDLL:
     L.uavb_rollout_targets_f64.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_double, c_void_p, c_int, c_void_p]
     L.uavb_rollout_f32.argtypes = [POINTER(RolloutArgs), c_void_p]
     L.uavb_rollout_f64.argtypes = [POINTER(RolloutArgs), c_void_p]
+    L.uavb_table_targets_f64.argtypes = [c_void_p, c_longlong, c_void_p, c_void_p]
+    L.uavb_rollout_tables_f32.argtypes = [POINTER(RolloutArgs), POINTER(TableSet), c_void_p]
     L.uavb_vehicle_defaults.argtypes = [POINTER(Vehicle)]
     L.uavb_vehicle_defaults.restype = None
     L.uavb_stage_f32.argtypes = [POINTER(StageArgs), c_void_p]

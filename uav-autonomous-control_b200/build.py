@@ -18,7 +18,7 @@ ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 LIBDIR = os.path.join(PKG, "lib")
 LIB = os.path.join(LIBDIR, "libuavb.so")
-SOURCES = ["capi.cu", "minsnap_kernels.cu", "minsnap_correct.cu", "rollout_kernels.cu", "rollout_sliced.cu", "rollout_log.cu", "rollout_traj.cu", "rollout_scalar.cu", "rollout_f64.cu", "stage_kernels.cu",
+SOURCES = ["capi.cu", "minsnap_kernels.cu", "minsnap_correct.cu", "rollout_kernels.cu", "rollout_sliced.cu", "rollout_log.cu", "rollout_traj.cu", "rollout_tables.cu", "rollout_tables_log.cu", "rollout_scalar.cu", "rollout_f64.cu", "stage_kernels.cu",
            "mc_kernels.cu", "host_api.cu", "rrt_kernels.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--extended-lambda",
               "-Xcompiler", "-fPIC"]

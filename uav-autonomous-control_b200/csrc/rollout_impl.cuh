@@ -330,6 +330,26 @@ __device__ __forceinline__ void mission_view(MissionView& m, const RolloutDev<fl
   }
 }
 
+// Caller-supplied trajectory tables, one per rollout (uavb_rollout_tables_f32 with shared_rows = 0): rollout i flies the
+// TargetRow records [offsets[t], offsets[t + 1]) of table t = table_index[i] (t = i when table_index is NULL).
+struct TableSetDev {
+  const TargetRow* rows;
+  const long long* offsets;
+  const int* table_index;
+};
+
+// The mission view of a per-rollout table: only trows / n_trows are read (PairTarget<kTargetPerRollout>); the cursor row is
+// relative to the table, so the carry block resumes with the same table set.
+__device__ __forceinline__ void table_view(MissionView& m, const TableSetDev& ts, long long i) {
+  const long long t = ts.table_index ? (long long)ts.table_index[i] : i;
+  const long long first = ts.offsets[t];
+  m.coeffs = nullptr; m.rows = nullptr; m.table = nullptr; m.yaw0 = nullptr;
+  m.seg_begin = 0; m.seg_count = 0; m.dt_outer = 0.0;
+  m.trows = ts.rows + first;
+  m.n_trows = (int)(ts.offsets[t + 1] - first);
+  m.cache = nullptr; m.cache_stride = 0;
+}
+
 // Final outputs of one drone (state, metrics) -- shared by the pair path; same values as drone_slice's epilogue.
 __device__ __forceinline__ void write_outputs(const uavb_rollout_args& a, long long i, Drone<float>& d, const Cursor<float>& c,
                                               const Accum<float>& acc, bool log) {
@@ -367,9 +387,11 @@ __device__ __forceinline__ void write_outputs(const uavb_rollout_args& a, long l
 // drone_slice.  When B is odd the last pair's second lane re-flies the first drone and writes nothing.
 // LOG: 0 = no state log, 1 = per-thread streaming stores (PairLog), 2 = staged tensor stores (PairLogTma, `maps` required),
 // 3 = the gated position list of the viewer (PairTrajLog; its state rides in the carry block between slices).
-template <int LOG, bool MC, bool TABLE, bool LAG>
+// MODE: where the set-points come from (kTargetFly / kTargetShared / kTargetPerRollout, rollout_pair.cuh); the last needs `tabs`.
+template <int LOG, bool MC, int MODE, bool LAG>
 __device__ __forceinline__ void pair_slice(const RolloutDev<float>& p, long long j, int n_ticks, bool from_carry, bool to_carry,
-                                           bool finish, int launch_tick0, const LogTma* maps = nullptr, bool first_slice = true) {
+                                           bool finish, int launch_tick0, const LogTma* maps = nullptr, bool first_slice = true,
+                                           const TableSetDev* tabs = nullptr) {
   const uavb_rollout_args& a = p.a;
   const long long B = a.B;
   const long long i0 = 2 * j;
@@ -397,8 +419,13 @@ __device__ __forceinline__ void pair_slice(const RolloutDev<float>& p, long long
   zip_veho(vo, va, vb);
 
   MissionView ma, mb;
-  mission_view(ma, p, i0, 2 * (int)threadIdx.x, 2 * (int)blockDim.x);
-  mission_view(mb, p, i1, 2 * (int)threadIdx.x + 1, 2 * (int)blockDim.x);
+  if constexpr (MODE == kTargetPerRollout) {
+    table_view(ma, *tabs, i0);
+    table_view(mb, *tabs, i1);
+  } else {
+    mission_view(ma, p, i0, 2 * (int)threadIdx.x, 2 * (int)blockDim.x);
+    mission_view(mb, p, i1, 2 * (int)threadIdx.x + 1, 2 * (int)blockDim.x);
+  }
 
   Drone2 d;
   Cursor<float> c[2];
@@ -427,8 +454,8 @@ __device__ __forceinline__ void pair_slice(const RolloutDev<float>& p, long long
   auto fly = [&](const auto& oa, const auto& ob) {
     auto with_log = [&](auto& lg) {
       const Ground gr{a.ground_on, a.ground_z};
-      if constexpr (MC) rollout_run_pair<TABLE, LAG>(d, c, acc, u, va, vb, v2, vo, ma, mb, tick0, n_ticks, a.inner_per_outer, oa, ob, lg, gr);
-      else rollout_run_pair<TABLE, LAG>(d, c, acc, u, va, vb, p.vp, vo, ma, mb, tick0, n_ticks, a.inner_per_outer, oa, ob, lg, gr);
+      if constexpr (MC) rollout_run_pair<MODE, LAG>(d, c, acc, u, va, vb, v2, vo, ma, mb, tick0, n_ticks, a.inner_per_outer, oa, ob, lg, gr);
+      else rollout_run_pair<MODE, LAG>(d, c, acc, u, va, vb, p.vp, vo, ma, mb, tick0, n_ticks, a.inner_per_outer, oa, ob, lg, gr);
     };
     if constexpr (LOG == 3) {
       PairTrajLog lg;
@@ -553,8 +580,8 @@ __device__ __forceinline__ int ld_acquire_gpu(const int* p) {
 }
 __device__ __forceinline__ void st_release_gpu(int* p, int v) { asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
 
-template <bool MC, bool TABLE, int LOG, bool LAG>
-__device__ __forceinline__ void sliced_body(const RolloutDev<float>& p, const SliceSched& sch, const LogTma* maps) {
+template <bool MC, int MODE, int LOG, bool LAG>
+__device__ __forceinline__ void sliced_body(const RolloutDev<float>& p, const SliceSched& sch, const LogTma* maps, const TableSetDev* tabs = nullptr) {
   extern __shared__ __align__(128) float s_boxes[];
   __shared__ int s_item;
   stage_shared_boxes(p.a, s_boxes);
@@ -577,7 +604,7 @@ __device__ __forceinline__ void sliced_body(const RolloutDev<float>& p, const Sl
       const bool last = c == sch.n_chunks - 1;
       const int t0 = sch.begin(c);
       const int ticks = last ? p.a.n_ticks - t0 : sch.begin(c + 1) - t0;
-      pair_slice<LOG, MC, TABLE, LAG>(p, j, ticks, c > 0 || p.a.resume != 0, !last || sch.final_carry != 0, last, t0, maps, c == 0);
+      pair_slice<LOG, MC, MODE, LAG>(p, j, ticks, c > 0 || p.a.resume != 0, !last || sch.final_carry != 0, last, t0, maps, c == 0, tabs);
     }
     __threadfence();
     __syncthreads();
@@ -587,7 +614,7 @@ __device__ __forceinline__ void sliced_body(const RolloutDev<float>& p, const Sl
 
 template <bool MC, bool TABLE, bool LOG, bool LAG>
 __global__ void __maxnreg__(kRolloutPairRegs) rollout_sliced_kernel(const __grid_constant__ RolloutDev<float> p, const SliceSched sch) {
-  sliced_body<MC, TABLE, LOG ? 1 : 0, LAG>(p, sch, nullptr);
+  sliced_body<MC, TABLE ? kTargetShared : kTargetFly, LOG ? 1 : 0, LAG>(p, sch, nullptr);
 }
 
 // One drone per thread at 128 registers, 16 one-warp CTAs per SM: the round-1 kernel, kept for metrics-only rollouts with PER-ROLLOUT
@@ -631,14 +658,32 @@ __global__ void __maxnreg__(kRolloutRegs) rollout_sliced_scalar_kernel(const __g
 // Metrics + the gated position list of the viewer (PairTrajLog); one-warp CTAs like the metrics-only kernel.
 template <bool MC, bool TABLE, bool LAG>
 __global__ void __maxnreg__(kRolloutPairRegs) rollout_sliced_traj_kernel(const __grid_constant__ RolloutDev<float> p, const SliceSched sch) {
-  sliced_body<MC, TABLE, 3, LAG>(p, sch, nullptr);
+  sliced_body<MC, TABLE ? kTargetShared : kTargetFly, 3, LAG>(p, sch, nullptr);
 }
 
 // The state log through staged tensor stores (PairLogTma); `maps` lives in the kernel parameter space, where the TMA unit reads it.
 template <bool MC, bool TABLE, bool LAG>
 __global__ void __maxnreg__(kRolloutPairRegs) rollout_sliced_tma_kernel(const __grid_constant__ RolloutDev<float> p, const SliceSched sch,
                                                                          const __grid_constant__ LogTma maps) {
-  sliced_body<MC, TABLE, 2, LAG>(p, sch, &maps);
+  sliced_body<MC, TABLE ? kTargetShared : kTargetFly, 2, LAG>(p, sch, &maps);
+}
+
+// The same three families flying caller-supplied tables, one per rollout (kTargetPerRollout): metrics only or per-thread log
+// stores, the flown-path list, staged tensor stores.  `ts` lives in the kernel parameter space like `maps`.
+template <bool MC, bool LOG, bool LAG>
+__global__ void __maxnreg__(kRolloutPairRegs) rollout_sliced_tables_kernel(const __grid_constant__ RolloutDev<float> p, const SliceSched sch,
+                                                                            const __grid_constant__ TableSetDev ts) {
+  sliced_body<MC, kTargetPerRollout, LOG ? 1 : 0, LAG>(p, sch, nullptr, &ts);
+}
+template <bool MC, bool LAG>
+__global__ void __maxnreg__(kRolloutPairRegs) rollout_sliced_tables_traj_kernel(const __grid_constant__ RolloutDev<float> p, const SliceSched sch,
+                                                                                 const __grid_constant__ TableSetDev ts) {
+  sliced_body<MC, kTargetPerRollout, 3, LAG>(p, sch, nullptr, &ts);
+}
+template <bool MC, bool LAG>
+__global__ void __maxnreg__(kRolloutPairRegs) rollout_sliced_tables_tma_kernel(const __grid_constant__ RolloutDev<float> p, const SliceSched sch,
+                                                                                const __grid_constant__ LogTma maps, const __grid_constant__ TableSetDev ts) {
+  sliced_body<MC, kTargetPerRollout, 2, LAG>(p, sch, &maps, &ts);
 }
 
 
@@ -647,6 +692,11 @@ void launch_rollout_sliced(bool mc, bool table, int grid, size_t smem, cudaStrea
 void launch_rollout_sliced_log(bool mc, bool table, int grid, size_t smem, cudaStream_t st, const RolloutDev<float>& p, const SliceSched& sch,
                                const LogTma* maps);      // maps != nullptr: staged tensor stores
 void launch_rollout_sliced_traj(bool mc, bool table, int grid, size_t smem, cudaStream_t st, const RolloutDev<float>& p, const SliceSched& sch);
+// per-rollout caller tables (rollout_tables.cu: metrics only / flown-path list; rollout_tables_log.cu: state log, maps as above)
+void launch_rollout_tables(bool mc, bool traj, int grid, size_t smem, cudaStream_t st, const RolloutDev<float>& p, const SliceSched& sch,
+                           const TableSetDev& ts);
+void launch_rollout_tables_log(bool mc, int grid, size_t smem, cudaStream_t st, const RolloutDev<float>& p, const SliceSched& sch,
+                               const LogTma* maps, const TableSetDev& ts);
 void launch_rollout_sliced_scalar(bool mc, int grid, size_t smem, cudaStream_t st, const RolloutDev<float>& p, const SliceSched& sch);
 void launch_rollout_f64(bool log, bool mc, int grid, size_t smem, cudaStream_t st, const RolloutDev<double>& p);
 

@@ -62,14 +62,23 @@ __global__ void __launch_bounds__(128) target_heading_kernel(const float2* __res
   out[g].yc = h.x; out[g].ys = h.y;
 }
 
-static int check_args(const uavb_rollout_args* a, bool f64) {
+// tables: the arguments of uavb_rollout_tables_f32, where the set-points come from a uavb_table_set and every mission-segment field
+// must be NULL / 0.
+static int check_args(const uavb_rollout_args* a, bool f64, bool tables = false) {
   UAVB_REQUIRE(a != nullptr, "rollout: args is NULL");
   UAVB_REQUIRE(a->B >= 0 && a->n_ticks >= 0, "rollout: B and n_ticks must be >= 0");
   UAVB_REQUIRE(a->inner_per_outer >= 1, "rollout: inner_per_outer must be >= 1");
-  UAVB_REQUIRE(a->seg_coeffs && a->seg_rows && a->seg_table && a->seg_yaw0, "rollout: mission segment arrays are required");
-  UAVB_REQUIRE((a->mission_seg_begin == nullptr) == (a->mission_seg_count == nullptr),
-               "rollout: mission_seg_begin and mission_seg_count must be given together");
-  UAVB_REQUIRE(a->mission_seg_begin != nullptr || a->n_seg_shared >= 1, "rollout: n_seg_shared must be >= 1 for a shared mission");
+  if (tables) {
+    UAVB_REQUIRE(!a->seg_coeffs && !a->seg_rows && !a->seg_table && !a->seg_yaw0 && !a->mission_seg_begin && !a->mission_seg_count &&
+                     a->n_seg_shared == 0 && !a->shared_targets && a->n_target_rows == 0,
+                 "rollout_tables: the mission-segment fields of args (seg_*, mission_seg_*, n_seg_shared, shared_targets, n_target_rows) "
+                 "must be NULL / 0");
+  } else {
+    UAVB_REQUIRE(a->seg_coeffs && a->seg_rows && a->seg_table && a->seg_yaw0, "rollout: mission segment arrays are required");
+    UAVB_REQUIRE((a->mission_seg_begin == nullptr) == (a->mission_seg_count == nullptr),
+                 "rollout: mission_seg_begin and mission_seg_count must be given together");
+    UAVB_REQUIRE(a->mission_seg_begin != nullptr || a->n_seg_shared >= 1, "rollout: n_seg_shared must be >= 1 for a shared mission");
+  }
   UAVB_REQUIRE(a->resume || a->start != nullptr, "rollout: start is required when resume = 0");
   UAVB_REQUIRE(a->start_stride == 0 || a->start_stride == 3, "rollout: start_stride must be 0 or 3");
   UAVB_REQUIRE(a->goal == nullptr || a->goal_stride == 0 || a->goal_stride == 3, "rollout: goal_stride must be 0 or 3");
@@ -83,7 +92,7 @@ static int check_args(const uavb_rollout_args* a, bool f64) {
   UAVB_REQUIRE(a->traj_out == nullptr || (a->traj_max_samples >= 1 && a->traj_interval >= 0.0), "rollout: traj_out needs traj_max_samples >= 1 and traj_interval >= 0");
   UAVB_REQUIRE(a->n_obs >= 0 && a->n_obs <= 1024, "rollout: n_obs out of range");
   UAVB_REQUIRE(a->n_obs == 0 || (a->aabbs != nullptr && a->n_obs_sets >= 1), "rollout: n_obs > 0 needs aabbs and n_obs_sets >= 1");
-  UAVB_REQUIRE(a->dt_outer > 0.0 && a->veh.dt > 0.0 && a->veh.mass > 0.0, "rollout: dt_outer, veh.dt and veh.mass must be positive");
+  UAVB_REQUIRE((tables || a->dt_outer > 0.0) && a->veh.dt > 0.0 && a->veh.mass > 0.0, "rollout: dt_outer, veh.dt and veh.mass must be positive");
   UAVB_REQUIRE(a->shared_targets == nullptr || (a->mission_seg_begin == nullptr && a->n_target_rows >= 1),
                "rollout: shared_targets needs a shared mission and n_target_rows >= 1");
   return UAVB_OK;
@@ -101,8 +110,9 @@ struct StreamScratch {
   }
 };
 
-template <class R> static int launch_rollout(const uavb_rollout_args* a, void* stream) {
-  int rc = check_args(a, sizeof(R) == 8);
+// tabs != nullptr: per-rollout caller tables (fp32 only).  checked: the caller validated the arguments (uavb_rollout_tables_f32).
+template <class R> static int launch_rollout(const uavb_rollout_args* a, void* stream, const TableSetDev* tabs = nullptr, bool checked = false) {
+  int rc = checked ? UAVB_OK : check_args(a, sizeof(R) == 8);
   if (rc) return rc;
   rc = require_device();
   if (rc) return rc;
@@ -125,7 +135,7 @@ template <class R> static int launch_rollout(const uavb_rollout_args* a, void* s
   p.vehp_cache = nullptr;
   p.vehp_stride = 0;
   const bool from_table = a->shared_targets != nullptr && a->mission_seg_begin == nullptr;
-  if (!from_table && sizeof(R) == 4) {                            // fp32 kernels stage the current spline in shared memory
+  if (!from_table && tabs == nullptr && sizeof(R) == 4) {                            // fp32 kernels stage the current spline in shared memory
     smem = (smem + 7) / 8 * 8;
     p.coeff_cache_offset = (int)(smem / 8);
     smem += sizeof(double) * 24 * per_cta;
@@ -133,6 +143,7 @@ template <class R> static int launch_rollout(const uavb_rollout_args* a, void* s
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const bool mc_any = a->mc_mass || a->mc_inertia || a->mc_gains || a->mc_wind;
   if constexpr (sizeof(R) == 8) {                      // validation build
+    (void)tabs;
     launch_rollout_f64(log, mc_any, grid, smem, st, p);
   } else {
     int sms = 0;
@@ -230,7 +241,9 @@ template <class R> static int launch_rollout(const uavb_rollout_args* a, void* s
         smem += sizeof(float) * kLogTmaWarpFloats * (kRolloutThreadsLog / 32);
       }
     }
-    if (log) launch_rollout_sliced_log(mc_any, from_table, pgrid, smem, st, *reinterpret_cast<RolloutDev<float>*>(&p), sch, tma_log ? &maps : nullptr);
+    if (tabs && log) launch_rollout_tables_log(mc_any, pgrid, smem, st, *reinterpret_cast<RolloutDev<float>*>(&p), sch, tma_log ? &maps : nullptr, *tabs);
+    else if (tabs) launch_rollout_tables(mc_any, a->traj_out != nullptr, pgrid, smem, st, *reinterpret_cast<RolloutDev<float>*>(&p), sch, *tabs);
+    else if (log) launch_rollout_sliced_log(mc_any, from_table, pgrid, smem, st, *reinterpret_cast<RolloutDev<float>*>(&p), sch, tma_log ? &maps : nullptr);
     else if (scalar32) launch_rollout_sliced_scalar(mc_any, pgrid, smem, st, *reinterpret_cast<RolloutDev<float>*>(&p), sch);
     else if (a->traj_out) launch_rollout_sliced_traj(mc_any, from_table, pgrid, smem, st, *reinterpret_cast<RolloutDev<float>*>(&p), sch);
     else launch_rollout_sliced(mc_any, from_table, pgrid, smem, st, *reinterpret_cast<RolloutDev<float>*>(&p), sch);
@@ -239,7 +252,63 @@ template <class R> static int launch_rollout(const uavb_rollout_args* a, void* s
   return UAVB_OK;
 }
 
+// Caller tables -> set-point rows (uavb_table_targets_f64), one thread per row: x y z copied, v / a rounded once to fp32, the yaw
+// column as the heading direction (cos, sin) formed in fp64 (TrajectoryController feeds row[9] to the yaw controller, main.py:58,
+// and a direction makes psi and psi + 2 pi k the same set-point, as wrap_to_pi(wrap_to_2pi(psi_des) - psi) does, controller.py:156-168).
+__global__ void __launch_bounds__(128) table_targets_kernel(const double* __restrict__ tables, long long n_rows, TargetRow* __restrict__ out) {
+  const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (g >= n_rows) return;
+  const double* r = tables + g * 11;
+  TargetRow t;
+  t.x = r[0]; t.y = r[1]; t.z = r[2];
+  t.vx = (float)r[3]; t.vy = (float)r[4]; t.vz = (float)r[5];
+  t.ax = (float)r[6]; t.ay = (float)r[7]; t.az = (float)r[8];
+  const double yaw = r[9];
+  t.yc = (float)cos(yaw); t.ys = (float)sin(yaw);
+  out[g] = t;
+}
+
 }  // namespace uavb
+
+extern "C" int uavb_table_targets_f64(const double* tables, long long n_rows, void* targets_out, void* stream) {
+  using namespace uavb;
+  UAVB_REQUIRE(tables && targets_out, "table_targets: NULL pointer");
+  UAVB_REQUIRE(n_rows >= 0, "table_targets: n_rows must be >= 0");
+  int rc = require_device();
+  if (rc) return rc;
+  if (n_rows == 0) return UAVB_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const long long blocks = (n_rows + 127) / 128;
+  UAVB_REQUIRE(blocks <= 0x7fffffffLL, "table_targets: too many rows");
+  table_targets_kernel<<<(unsigned)blocks, 128, 0, st>>>(tables, n_rows, static_cast<TargetRow*>(targets_out));
+  UAVB_CUDA_OK(cudaGetLastError());
+  return UAVB_OK;
+}
+
+extern "C" int uavb_rollout_tables_f32(const uavb_rollout_args* args, const uavb_table_set* tables, void* stream) {
+  using namespace uavb;
+  int rc = check_args(args, false, true);
+  if (rc) return rc;
+  UAVB_REQUIRE(tables != nullptr && tables->rows != nullptr, "rollout_tables: tables and tables->rows are required");
+  UAVB_REQUIRE(tables->shared_rows >= 0, "rollout_tables: shared_rows must be >= 0");
+  if (tables->shared_rows > 0) {
+    UAVB_REQUIRE(tables->offsets == nullptr && tables->table_index == nullptr,
+                 "rollout_tables: a shared table (shared_rows > 0) takes no offsets and no table_index");
+  } else {
+    UAVB_REQUIRE(tables->n_tables >= 1 && tables->offsets != nullptr, "rollout_tables: per-rollout tables need n_tables >= 1 and offsets");
+    UAVB_REQUIRE(tables->table_index != nullptr || tables->n_tables == args->B || args->B == 0,
+                 "rollout_tables: without table_index rollout b flies table b (n_tables == B)");
+  }
+  uavb_rollout_args a = *args;
+  a.dt_outer = a.veh.dt * a.inner_per_outer;               // CascadedController.dt of the table's outer period (main.py:97)
+  if (tables->shared_rows > 0) {                           // the shared-mission table kernels, unchanged
+    a.shared_targets = tables->rows;
+    a.n_target_rows = tables->shared_rows;
+    return launch_rollout<float>(&a, stream, nullptr, true);
+  }
+  const TableSetDev ts{static_cast<const TargetRow*>(tables->rows), tables->offsets, tables->table_index};
+  return launch_rollout<float>(&a, stream, &ts, true);
+}
 
 extern "C" int uavb_rollout_targets_f64(const double* seg_coeffs, const int* seg_rows, const int* seg_table, const double* seg_yaw0, int n_seg,
                                         double dt_outer, void* targets_out, int n_rows, void* stream) {

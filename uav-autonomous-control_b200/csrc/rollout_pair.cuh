@@ -143,10 +143,27 @@ struct NoPairLog {
   UAVB_DEV void tick(const Drone2&) {}
 };
 
+// Where a pair's set-points come from (a compile-time switch of the kernel, so each body carries only its own code):
+//   kTargetFly         each lane evaluates its own mission's splines in fp64 (MissionView cursor);
+//   kTargetShared      one precomputed TargetRow table for every rollout (MissionView::trows), one row serves both lanes;
+//   kTargetPerRollout  each lane reads its own precomputed table (MissionView::trows / n_trows of the lane), e.g. caller-supplied
+//                      (N, 11) trajectory tables converted by uavb_table_targets_f64.
+enum : int { kTargetFly = 0, kTargetShared = 1, kTargetPerRollout = 2 };
+
+// Per-rollout tables: prefetch each lane's row of the NEXT outer period into L1 (as the shared-table body does for its one row),
+// and ticks per iteration of their metrics-only bodies (tools/table_probe.py measures both against the alternatives).
+#ifndef UAVB_TABLES_PREFETCH
+#define UAVB_TABLES_PREFETCH 1
+#endif
+#ifndef UAVB_TABLES_TICK_UNROLL
+#define UAVB_TABLES_TICK_UNROLL UAVB_TICK_UNROLL
+#endif
+constexpr int kTablesTickUnroll = UAVB_TABLES_TICK_UNROLL;
+
 // Set-points of the coming outer period and the position errors (set-point - position, fp64, rounded once): one table row
-// for both lanes of a shared mission, otherwise each lane's own cursor.
-template <bool TABLE> struct PairTarget;
-template <> struct PairTarget<true> {
+// for both lanes of a shared mission, otherwise each lane's own cursor or table.
+template <int MODE> struct PairTarget;
+template <> struct PairTarget<kTargetShared> {
   typedef float T;
   static UAVB_DEV void fetch(const Drone2& d, Cursor<float> (&c)[2], const MissionView& ma, const MissionView&, Target2<float>& t2, V2& ex, V2& ey, V2& ez) {
     Target<float> t;
@@ -163,7 +180,7 @@ template <> struct PairTarget<true> {
     ez = make_float2((float)(t.z - d.pz[0]), (float)(t.z - d.pz[1]));
   }
 };
-template <> struct PairTarget<false> {
+template <> struct PairTarget<kTargetFly> {
   typedef V2 T;
   static UAVB_DEV void fetch(const Drone2& d, Cursor<float> (&c)[2], const MissionView& ma, const MissionView& mb, Target2<V2>& t2, V2& ex, V2& ey, V2& ez) {
     Target<float> ta, tb;
@@ -171,6 +188,30 @@ template <> struct PairTarget<false> {
     cursor_advance(&c[0].seg, &c[0].row, ma);
     cursor_target<float>(c[1], mb, &tb);
     cursor_advance(&c[1].seg, &c[1].row, mb);
+    t2.vx = make_float2(ta.vx, tb.vx); t2.vy = make_float2(ta.vy, tb.vy); t2.vz = make_float2(ta.vz, tb.vz);
+    t2.ax = make_float2(ta.ax, tb.ax); t2.ay = make_float2(ta.ay, tb.ay); t2.az = make_float2(ta.az, tb.az);
+    t2.yc = make_float2(ta.yc, tb.yc); t2.ys = make_float2(ta.ys, tb.ys);
+    ex = make_float2((float)(ta.x - d.px[0]), (float)(tb.x - d.px[1]));
+    ey = make_float2((float)(ta.y - d.py[0]), (float)(tb.y - d.py[1]));
+    ez = make_float2((float)(ta.z - d.pz[0]), (float)(tb.z - d.pz[1]));
+  }
+};
+template <> struct PairTarget<kTargetPerRollout> {
+  typedef V2 T;
+  static UAVB_DEV void fetch(const Drone2& d, Cursor<float> (&c)[2], const MissionView& ma, const MissionView& mb, Target2<V2>& t2, V2& ex, V2& ey, V2& ez) {
+    Target<float> ta, tb;
+    table_target<float>(ma.trows, c[0].row, &ta);
+    if (c[0].row + 1 < ma.n_trows) ++c[0].row;               // index clamp of main.py:61, with the lane's own row count
+    table_target<float>(mb.trows, c[1].row, &tb);
+    if (c[1].row + 1 < mb.n_trows) ++c[1].row;
+#if UAVB_TABLES_PREFETCH
+    const char* na = reinterpret_cast<const char*>(ma.trows + c[0].row);
+    const char* nb = reinterpret_cast<const char*>(mb.trows + c[1].row);
+    asm volatile("prefetch.global.L1 [%0];" ::"l"(na));
+    asm volatile("prefetch.global.L1 [%0];" ::"l"(na + sizeof(TargetRow) - 4));
+    asm volatile("prefetch.global.L1 [%0];" ::"l"(nb));
+    asm volatile("prefetch.global.L1 [%0];" ::"l"(nb + sizeof(TargetRow) - 4));
+#endif
     t2.vx = make_float2(ta.vx, tb.vx); t2.vy = make_float2(ta.vy, tb.vy); t2.vz = make_float2(ta.vz, tb.vz);
     t2.ax = make_float2(ta.ax, tb.ax); t2.ay = make_float2(ta.ay, tb.ay); t2.az = make_float2(ta.az, tb.az);
     t2.yc = make_float2(ta.yc, tb.yc); t2.ys = make_float2(ta.ys, tb.ys);
@@ -226,7 +267,8 @@ template <int L, class OBST> UAVB_DEV void pair_hit(const Drone2& d, Accum<float
 // LAG (thrust_frame_lag of the launch) is a compile-time switch of the kernel: one stretch body per (kernel, watch) keeps the
 // instruction footprint of a warp's working set inside the instruction cache (ncu: with all four (watch, lag) bodies in one kernel
 // the per-rollout-mission workload spent as long waiting for instructions as for operands).
-template <bool TABLE, bool LAG, class VP2, class OBST, class LOG>
+// MODE: kTargetFly / kTargetShared / kTargetPerRollout (PairTarget above).
+template <int MODE, bool LAG, class VP2, class OBST, class LOG>
 UAVB_DEV void rollout_run_pair(Drone2& d, Cursor<float> (&c)[2], Accum<float> (&a)[2], const VehU<float>& u, const VehP<float>& va,
                                const VehP<float>& vb, const VP2& v2, const VehO2& vo, const MissionView& ma, const MissionView& mb, int tick0,
                                int n_ticks, int freq, const OBST& oa, const OBST& ob, LOG& logger, const Ground gr = Ground{0, 0.0}) {
@@ -235,9 +277,9 @@ UAVB_DEV void rollout_run_pair(Drone2& d, Cursor<float> (&c)[2], Accum<float> (&
   const V2 acc_max = make_float2(va.acc_max, vb.acc_max);
   while (k < n_ticks) {
     if (c[0].phase == 0) {
-      Target2<typename PairTarget<TABLE>::T> t;
+      Target2<typename PairTarget<MODE>::T> t;
       V2 ex, ey, ez;
-      PairTarget<TABLE>::fetch(d, c, ma, mb, t, ex, ey, ez);    // the position is folded here (d.dx = 0)
+      PairTarget<MODE>::fetch(d, c, ma, mb, t, ex, ey, ez);    // the position is folded here (d.dx = 0)
       c[0].ex = ex.x; c[1].ex = ex.y; c[0].ey = ey.x; c[1].ey = ey.y; c[0].ez = ez.x; c[1].ez = ez.y;
       outer_update_pair(d, u, vo, t, ex, ey, ez);
     }
@@ -249,8 +291,10 @@ UAVB_DEV void rollout_run_pair(Drone2& d, Cursor<float> (&c)[2], Accum<float> (&
       // two ticks per iteration (the tail of one tick overlaps the head of the next: +2 % on the table-driven headline workload)
       // only where the instruction footprint allows it: the watching bodies carry the per-tick box tests, and kernels that
       // evaluate the set-points on the fly carry two inlined fp64 evaluations per period -- unrolled, BASELINE configs[3]
-      // waits for instruction fetches and runs 10 % slower (measured)
-#pragma unroll((kWatch || !TABLE) ? 1 : kTickUnroll)
+      // waits for instruction fetches and runs 10 % slower (measured).  Per-rollout tables unroll only without a state log: with
+      // Monte-Carlo overrides and per-thread log stores the unrolled body no longer fits 255 registers (ptxas spills), and a
+      // logging launch is bound by its HBM stores anyway.
+#pragma unroll((kWatch || MODE == kTargetFly) ? 1 : MODE == kTargetShared ? kTickUnroll : LOG::kNormEveryTick ? 1 : kTablesTickUnroll)
       for (int j = 0; j < n; ++j) {
         inner_tick_pair<LOG::kNormEveryTick, LAG>(d, u, v2);
         if constexpr (kWatch) {

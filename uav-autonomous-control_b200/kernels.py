@@ -478,6 +478,113 @@ def rollout_targets(plan: MissionPlan, n_rows: Optional[int] = None) -> torch.Te
     return out
 
 
+# ------------------------------------------------------------------------------------------ caller tables
+@dataclass
+class TablePlan:
+    """Caller-supplied (N, 11) trajectory tables in the layout K2 reads (struct uavb_table_set, include/uavb.h): what
+    TrajectoryController(controller, quad, trajectory, frequency) flies (main.py:10-61), for every rollout of a batch."""
+    rows: torch.Tensor                           # [n_rows, 56] u8 set-point records (uavb_table_targets_f64), tables one after the other
+    rows_per_table: tuple                        # host: rows of every table (known from the input shapes)
+    last_position: torch.Tensor                  # [n_tables, 3] f64 position of every table's last row (the default goal)
+    offsets: Optional[torch.Tensor] = None       # [n_tables + 1] i64 first row of every table; None = ONE table flown by every rollout
+    table_index: Optional[torch.Tensor] = None   # [B] i32 table of every rollout; None = rollout b flies table b
+
+    @property
+    def shared(self) -> bool:
+        return self.offsets is None
+
+    @property
+    def n_tables(self) -> int:
+        return len(self.rows_per_table)
+
+    @property
+    def max_rows(self) -> int:
+        return max(self.rows_per_table)
+
+    def goals(self, B: int) -> torch.Tensor:
+        """The last row's position of every rollout's table: [3] for a shared table, else [B, 3]."""
+        if self.shared:
+            return self.last_position[0].contiguous()
+        if self.table_index is None:
+            if self.n_tables != B:
+                raise ValueError(f"{self.n_tables} tables without table_index need B = {self.n_tables}, got {B}")
+            return self.last_position
+        return self.last_position.index_select(0, self.table_index.long()).contiguous()
+
+
+def table_targets(tables: torch.Tensor) -> torch.Tensor:
+    """[n_rows, 11] f64 (tables packed one after the other) -> [n_rows, 56] u8 set-point records (uavb_table_targets_f64): x y z
+    as given, v / a rounded to fp32, the yaw column as its heading direction (cos, sin)."""
+    if tables.dim() != 2 or tables.shape[1] != 11:
+        raise ValueError(f"tables must have shape (n_rows, 11), got {tuple(tables.shape)}")
+    out = torch.empty((tables.shape[0], nat.TARGET_ROW_BYTES), dtype=torch.uint8, device=tables.device)
+    nat.on(tables.device).uavb_table_targets_f64(nat.ptr(tables, torch.float64, "tables"), int(tables.shape[0]), nat.ptr(out),
+                                                 nat.stream_ptr(tables.device))
+    return out
+
+
+def plan_tables(tables, table_index=None, device=None) -> TablePlan:
+    """Trajectory tables [x y z vx vy vz ax ay az yaw spline_id] for ``rollout``.
+
+    ``tables``: one (N, 11) table, a (T, N, 11) stack, or a sequence of (N_t, 11) tables of different lengths (arrays or tensors).
+    One (N, 11) table without ``table_index`` is flown by every rollout (the shared-table kernel); otherwise rollout b flies table
+    ``table_index[b]`` ([B] ints in [0, T)), or table b when ``table_index`` is None (then B = T).  Every table needs >= 1 row.
+    The yaw column is the set-point itself, as TrajectoryController uses it; spline_id is ignored."""
+    import numpy as np
+
+    def as_f64(t):
+        return t.detach().to(dtype=torch.float64) if isinstance(t, torch.Tensor) else torch.as_tensor(np.asarray(t, dtype=np.float64))
+
+    single, stack = False, None
+    if isinstance(tables, (torch.Tensor, np.ndarray)):
+        stack = as_f64(tables)
+        if stack.dim() == 2:
+            parts, single = [stack], True
+        elif stack.dim() == 3:
+            parts = list(stack.unbind(0))
+        else:
+            raise ValueError(f"tables must be (N, 11), (T, N, 11) or a sequence of (N_t, 11) tables, got shape {tuple(stack.shape)}")
+    else:
+        parts = [as_f64(t) for t in tables]
+    if not parts:
+        raise ValueError("no tables given")
+    for k, t in enumerate(parts):
+        if t.dim() != 2 or t.shape[1] != 11:
+            raise ValueError(f"table {k} must have shape (N, 11), got {tuple(t.shape)}")
+        if t.shape[0] < 1:
+            raise ValueError(f"table {k} has no rows")
+    if table_index is not None:
+        idx = table_index if isinstance(table_index, torch.Tensor) else torch.as_tensor(np.asarray(table_index))
+        if idx.dim() != 1 or idx.dtype.is_floating_point or idx.dtype == torch.bool:
+            raise ValueError("table_index must be a 1-D integer array of shape (B,)")
+        _check_index_range(idx, len(parts))
+    dev =torch.device(device) if device is not None else (parts[0].device if parts[0].is_cuda else _dev())
+    counts = tuple(int(t.shape[0]) for t in parts)
+    if len(parts) == 1:
+        packed = parts[0].to(dev).contiguous()
+    elif stack is not None:                                                    # a (T, N, 11) stack is already packed
+        packed = stack.to(dev).reshape(-1, 11).contiguous()
+    else:
+        packed = torch.cat([p.to(dev) for p in parts]).contiguous()
+    ends = torch.tensor(np.cumsum(counts) - 1, dtype=torch.int64, device=dev)
+    plan = TablePlan(table_targets(packed), counts, packed.index_select(0, ends)[:, :3].contiguous())
+    if single and table_index is None:
+        return plan
+    plan.offsets = torch.tensor(np.concatenate(([0], np.cumsum(counts))), dtype=torch.int64, device=dev)
+    if table_index is not None:
+        plan.table_index = idx.to(device=dev, dtype=torch.int32).contiguous()
+    return plan
+
+
+def _check_index_range(idx: torch.Tensor, n_tables: int) -> None:
+    """0 <= idx < n_tables: one reduction (on the device for a CUDA tensor, one read back)."""
+    if idx.numel() == 0:
+        return
+    lo, hi = torch.stack(torch.aminmax(idx)).tolist()
+    if lo < 0 or hi >= n_tables:
+        raise ValueError(f"table_index must lie in [0, {n_tables}), got values in [{lo}, {hi}]")
+
+
 # ------------------------------------------------------------------------------------------ K2
 @dataclass
 class RolloutResult:
@@ -490,7 +597,7 @@ class RolloutResult:
     traj_count: Optional[torch.Tensor] = None  # [B] i32 samples the reference would hold
 
 
-def rollout(plan: MissionPlan, B: int, n_ticks: int, *, start: torch.Tensor, goal: Optional[torch.Tensor] = None,
+def rollout(plan, B: int, n_ticks: int, *, start: torch.Tensor, goal: Optional[torch.Tensor] = None,
             vehicle: Optional[nat.Vehicle] = None, frequency: int = 10, mc_mass: Optional[torch.Tensor] = None,
             mc_inertia: Optional[torch.Tensor] = None, mc_gains: Optional[torch.Tensor] = None, mc_wind: Optional[torch.Tensor] = None,
             obstacles: Optional[torch.Tensor] = None, obstacle_set: Optional[torch.Tensor] = None, thrust_frame_lag: int = 1,
@@ -509,9 +616,14 @@ def rollout(plan: MissionPlan, B: int, n_ticks: int, *, start: torch.Tensor, goa
     ground_z: optional unilateral floor (NED; uavb.h ground_on / ground_z).  traj_max_samples > 0 also records the viewer's
     flown-path list (MujocoSimulation._record_actual_trajectory, mujoco_sim.py:201-218): positions every traj_interval seconds
     of simulation time while z <= traj_gate_z, into result.traj [traj_max_samples, 3, B] / result.traj_count [B].
+    ``plan``: a MissionPlan (waypoint missions), or a TablePlan (``plan_tables``: caller trajectory tables, one row per
+    ``frequency`` ticks; fp32 only).
     """
-    dev = plan.seg_coeffs.device
+    tables = isinstance(plan, TablePlan)
+    dev = plan.rows.device if tables else plan.seg_coeffs.device
     f64 = dtype == torch.float64
+    if tables and f64:
+        raise ValueError("trajectory tables fly in the fp32 rollout only (uavb_rollout_f64 takes waypoint missions)")
     odt = torch.float64 if f64 else torch.float32
     a = nat.RolloutArgs()
     a.B, a.n_ticks, a.inner_per_outer = int(B), int(n_ticks), int(frequency)
@@ -531,21 +643,36 @@ def rollout(plan: MissionPlan, B: int, n_ticks: int, *, start: torch.Tensor, goa
                            ("mc_wind", mc_wind, (3, B))):
         if t is not None and tuple(t.shape) != shape:
             raise ValueError(f"{name} must have shape {shape}, got {tuple(t.shape)}")
-    a.seg_coeffs = nat.ptr(plan.seg_coeffs, torch.float64, "seg_coeffs")
-    a.seg_rows = nat.ptr(plan.seg_rows, torch.int32, "seg_rows")
-    a.seg_table = nat.ptr(plan.seg_table, torch.int32, "seg_table")
-    a.seg_yaw0 = nat.ptr(plan.seg_yaw0, torch.float64, "seg_yaw0")
-    if plan.shared:
-        a.n_seg_shared = int(plan.n_seg_shared)
-        if plan.targets is not None and use_targets:
-            a.shared_targets = nat.ptr(plan.targets, torch.uint8, "targets")
-            a.n_target_rows = int(plan.targets.shape[0])
+    ts = nat.TableSet()
+    if tables:                                        # every mission-segment field stays NULL / 0 (uavb_rollout_tables_f32)
+        ts.rows = nat.ptr(plan.rows, torch.uint8, "rows")
+        if plan.shared:
+            ts.shared_rows = int(plan.rows.shape[0])
+        else:
+            ts.offsets = nat.ptr(plan.offsets, torch.int64, "offsets")
+            ts.n_tables = plan.n_tables
+            if plan.table_index is not None:
+                if plan.table_index.numel() != B:
+                    raise ValueError(f"table_index holds {plan.table_index.numel()} rollouts, B = {B}")
+                ts.table_index = nat.ptr(plan.table_index, torch.int32, "table_index")
+            elif plan.n_tables != B:
+                raise ValueError(f"{plan.n_tables} tables without table_index need B = {plan.n_tables}, got {B}")
     else:
-        if plan.seg_begin.numel() != B:
-            raise ValueError("plan holds per-rollout missions for a different batch size")
-        a.mission_seg_begin = nat.ptr(plan.seg_begin, torch.int32, "seg_begin")
-        a.mission_seg_count = nat.ptr(plan.seg_count, torch.int32, "seg_count")
-    a.dt_outer = float(plan.dt)
+        a.seg_coeffs = nat.ptr(plan.seg_coeffs, torch.float64, "seg_coeffs")
+        a.seg_rows = nat.ptr(plan.seg_rows, torch.int32, "seg_rows")
+        a.seg_table = nat.ptr(plan.seg_table, torch.int32, "seg_table")
+        a.seg_yaw0 = nat.ptr(plan.seg_yaw0, torch.float64, "seg_yaw0")
+        if plan.shared:
+            a.n_seg_shared = int(plan.n_seg_shared)
+            if plan.targets is not None and use_targets:
+                a.shared_targets = nat.ptr(plan.targets, torch.uint8, "targets")
+                a.n_target_rows = int(plan.targets.shape[0])
+        else:
+            if plan.seg_begin.numel() != B:
+                raise ValueError("plan holds per-rollout missions for a different batch size")
+            a.mission_seg_begin = nat.ptr(plan.seg_begin, torch.int32, "seg_begin")
+            a.mission_seg_count = nat.ptr(plan.seg_count, torch.int32, "seg_count")
+        a.dt_outer = float(plan.dt)
     a.start = nat.ptr(start, torch.float64, "start")
     a.start_stride = 0 if start.dim() == 1 else 3
     if goal is not None:
@@ -584,9 +711,12 @@ def rollout(plan: MissionPlan, B: int, n_ticks: int, *, start: torch.Tensor, goa
             res.traj_count = torch.zeros((B,), dtype=torch.int32, device=dev)
         a.traj_out, a.traj_count_out = nat.ptr(res.traj, torch.float32, "traj"), nat.ptr(res.traj_count, torch.int32, "traj_count")
         a.traj_max_samples, a.traj_gate_z, a.traj_interval = int(res.traj.shape[0]), float(traj_gate_z), float(traj_interval)
-    fn = nat.lib().uavb_rollout_f64 if f64 else nat.lib().uavb_rollout_f32
     with torch.cuda.device(dev):                      # the library works on the CURRENT device: make it the tensors' device
-        nat.check(fn(ctypes.byref(a), nat.stream_ptr(dev)), "uavb_rollout_f64" if f64 else "uavb_rollout_f32")
+        if tables:
+            nat.check(nat.lib().uavb_rollout_tables_f32(ctypes.byref(a), ctypes.byref(ts), nat.stream_ptr(dev)), "uavb_rollout_tables_f32")
+        else:
+            fn = nat.lib().uavb_rollout_f64 if f64 else nat.lib().uavb_rollout_f32
+            nat.check(fn(ctypes.byref(a), nat.stream_ptr(dev)), "uavb_rollout_f64" if f64 else "uavb_rollout_f32")
     return res
 
 

@@ -130,3 +130,37 @@ class BatchedSimulation:
                                log_stride=log_stride, want_state=want_state, ground_z=float(self.mission_waypoints[0][2]) if ground else None,
                                traj_max_samples=(n_ticks // int(round(self.ACTUAL_TRAJECTORY_SAMPLE_INTERVAL / q.dt)) + 1) if record_actual_trajectory else 0,
                                traj_gate_z=float(self.mission_waypoints[1][2]), traj_interval=self.ACTUAL_TRAJECTORY_SAMPLE_INTERVAL)
+
+    def fly_trajectory(self, trajectory, frequency: int = 10, n_ticks: Optional[int] = None, *, table_index=None, start=None, goal=None,
+                       gains: Optional[dict] = None, log_stride: int = 0, want_state: bool = True, record_actual_trajectory: bool = False,
+                       ground: bool = False):
+        """Fly caller-supplied (N, 11) trajectory tables [x y z vx vy vz ax ay az yaw spline_id] in one launch of the persistent
+        rollout kernel: ``TrajectoryController(controller, quad, trajectory, frequency)`` followed by ``step()`` over the table
+        (main.py:10-61) for every drone -- one row per ``frequency`` ticks, the index held at the last row.
+
+        ``trajectory``: one table flown by every drone, a (T, N, 11) stack or a sequence of (N_t, 11) tables with ``table_index``
+        (B,) choosing each drone's table (None: drone b flies table b), or a ``kernels.TablePlan``.  ``start``: [3] or (B, 3), default
+        the scene start; ``goal`` (for final_dist): default the last row's position of each drone's table; ``n_ticks``: default
+        ``frequency`` x the rows of the longest table.  Mass / inertia, ``gains`` and ``self.wind`` as in ``rollout()``.
+        Returns ``kernels.RolloutResult``."""
+        q = self.quad
+        dev = self.device
+        if isinstance(trajectory, kernels.TablePlan):
+            if table_index is not None:
+                raise ValueError("table_index belongs to the TablePlan (kernels.plan_tables)")
+            plan = trajectory
+        else:
+            plan = kernels.plan_tables(trajectory, table_index, device=dev)
+        if n_ticks is None:
+            n_ticks = frequency * plan.max_rows
+        start = torch.tensor(self.mission_waypoints[0], dtype=torch.float64, device=dev) if start is None else \
+            torch.as_tensor(start, dtype=torch.float64).to(dev).contiguous()
+        goal = plan.goals(self.batch) if goal is None else torch.as_tensor(goal, dtype=torch.float64).to(dev).contiguous()
+        veh, mc = q.vehicle_struct(self.batch, gains or {})
+        return kernels.rollout(plan, self.batch, n_ticks, start=start, goal=goal, vehicle=veh, frequency=frequency,
+                               mc_mass=mc.get("mc_mass"), mc_inertia=mc.get("mc_inertia"), mc_gains=mc.get("mc_gains"),
+                               mc_wind=st.soa(self.wind) if self.wind is not None else None,
+                               obstacles=self._obs if len(self.obstacles) else None, thrust_frame_lag=self.thrust_frame_lag,
+                               log_stride=log_stride, want_state=want_state, ground_z=float(self.mission_waypoints[0][2]) if ground else None,
+                               traj_max_samples=(n_ticks // int(round(self.ACTUAL_TRAJECTORY_SAMPLE_INTERVAL / q.dt)) + 1) if record_actual_trajectory else 0,
+                               traj_gate_z=float(self.mission_waypoints[1][2]), traj_interval=self.ACTUAL_TRAJECTORY_SAMPLE_INTERVAL)
