@@ -219,6 +219,58 @@ template <bool NORM, bool LAG, class VP> UAVB_DEV void inner_tick_pair(Drone2& d
   }
 }
 
+// The speculative tick (rollout_run_pair): inner_tick_pair<false, LAG> without its two rare paths and without a branch.  It always
+// keeps the unclipped mixer outputs and the tan-form quaternion map; a lane where the exact tick would take the rotor-limit path
+// (failed sufficient test) or the large-rotation path (|w|^2 >= small_rot_wn2) sets its bit in `rare`, and its state is then wrong.
+// Where no bit is set the tick ran exactly the rounded operations of inner_tick_pair<false, LAG>.  (Kept as a copy rather than a
+// template switch of inner_tick_pair, so that the kernels that do not speculate compile to the same code as before.)
+// Bits of `rare`: one for both paths unless a counting build (UAVB_SPEC_COUNT, development only) tells them apart.
+#ifndef UAVB_SPEC_COUNT
+#define UAVB_SPEC_COUNT 0
+#endif
+constexpr int kRareLimitBit = 0;
+constexpr int kRareRotBit = UAVB_SPEC_COUNT ? 1 : 0;
+template <bool LAG, class VP> UAVB_DEV void inner_tick_pair_spec(Drone2& d, const VehU<float>& u, const VP& v, unsigned& rare) {
+  const V2 yz = mul2(d.wy, d.wz), zx = mul2(d.wz, d.wx), xy = mul2(d.wx, d.wy);
+  // mixer butterfly of mix_and_limit_pair, its sufficient test recorded instead of branched on
+  const V2 pb = fma2(neg2(v.Jp), d.wx, fma2(v.Gx, yz, d.cp)), qb = fma2(neg2(v.Jq), d.wy, fma2(v.Gy, zx, d.cq));
+  const V2 rb = fma2(neg2(v.Jr), d.wz, fma2(v.Gz, xy, d.cr));
+  const V2 m1 = add2(pb, qb), m2 = sub2(pb, qb), t1 = add2(d.coll, rb), t2 = sub2(d.coll, rb);
+  const V2 need = add2(add2(abs2(pb), abs2(qb)), abs2(rb));
+  rare |= (unsigned)(!(need.x <= d.margin.x) | !(need.y <= d.margin.y)) << kRareLimitBit;
+  lag_toward_pair(d, u, sqrt2(add2(t1, m1)), sqrt2(sub2(t2, m2)), sqrt2(sub2(t1, m1)), sqrt2(add2(t2, m2)));
+  V2 ha, hb, hc;
+  half_axis_pair(d, ha, hb, hc);
+  const V2 ua = LAG ? d.zbx : ha, ub = LAG ? d.zby : hb, uc = LAG ? d.zbz : hc;
+  d.zbx = ha; d.zby = hb; d.zbz = hc;
+  // rotor sums (mujoco_sim.py:235-247): a = s0+s1, c = s0-s1, b = s2+s3, e = s2-s3 with s_i = w_i^2
+  const V2 s0 = mul2(d.om0, d.om0), s2 = mul2(d.om2, d.om2);
+  const V2 a = fma2(d.om1, d.om1, s0), c = fma2(neg2(d.om1), d.om1, s0);
+  const V2 b = fma2(d.om3, d.om3, s2), e = fma2(neg2(d.om3), d.om3, s2);
+  const V2 tot = add2(a, b), ty = sub2(a, b), tx = sub2(c, e), tzn = add2(c, e);
+  const V2 dvt2 = mul2(neg2(tot), v.kf_dt_over_m2);
+  // semi-implicit Euler: velocity increments formed first (thrust and gravity cancel inside them near hover), new rates
+  d.vx = add2(d.vx, fma2(ua, dvt2, v.dvx));
+  d.vy = add2(d.vy, fma2(ub, dvt2, v.dvy));
+  d.vz = add2(d.vz, fma2(neg2(uc), dvt2, fma2(0.5f, dvt2, v.dvz)));
+  d.wx = fma2(v.Wx, tx, fma2(v.Kx, yz, d.wx));
+  d.wy = fma2(v.Wy, ty, fma2(v.Ky, zx, d.wy));
+  d.wz = fma2(neg2(v.Wz), tzn, fma2(v.Kz, xy, d.wz));
+  d.dx = fma2(u.dt, d.vx, d.dx);
+  d.dy = fma2(u.dt, d.vy, d.dy);
+  d.dz = fma2(u.dt, d.vz, d.dz);
+  // attitude (see above): b = (h + (h^3/3) |w|^2) w
+  const V2 wn2 = fma2(d.wx, d.wx, fma2(d.wy, d.wy, mul2(d.wz, d.wz)));
+  const V2 sf = fma2(wn2, u.half_dt_cu3, u.half_dt);
+  const V2 bx = mul2(sf, d.wx), by = mul2(sf, d.wy), bz = mul2(sf, d.wz);
+  const V2 q0 = d.q0, q1 = d.q1, q2 = d.q2, q3 = d.q3;
+  rare |= (unsigned)(!(wn2.x < u.small_rot_wn2) | !(wn2.y < u.small_rot_wn2)) << kRareRotBit;
+  d.q0 = sub2(q0, fma2(q3, bz, fma2(q2, by, mul2(q1, bx))));
+  d.q1 = add2(q1, fma2(neg2(q3), by, fma2(q2, bz, mul2(q0, bx))));
+  d.q2 = add2(q2, fma2(q3, bx, fma2(neg2(q1), bz, mul2(q0, by))));
+  d.q3 = add2(q3, fma2(neg2(q2), bx, fma2(q1, by, mul2(q0, bz))));
+}
+
 // ---------------------------------------------------------------------------------------------
 // 100 Hz outer loop of the pair: TrajectoryController._update_outer_loop (main.py:47-61) = altitude (controller.py:26-56),
 // lateral (:58-97), roll/pitch (:132-154), yaw (:156-168) on the fresh state, stage by stage as outer_update<float>.

@@ -391,7 +391,7 @@ __device__ __forceinline__ void write_outputs(const uavb_rollout_args& a, long l
 template <int LOG, bool MC, int MODE, bool LAG>
 __device__ __forceinline__ void pair_slice(const RolloutDev<float>& p, long long j, int n_ticks, bool from_carry, bool to_carry,
                                            bool finish, int launch_tick0, const LogTma* maps = nullptr, bool first_slice = true,
-                                           const TableSetDev* tabs = nullptr) {
+                                           const TableSetDev* tabs = nullptr, int spec_exact = 0) {
   const uavb_rollout_args& a = p.a;
   const long long B = a.B;
   const long long i0 = 2 * j;
@@ -454,8 +454,17 @@ __device__ __forceinline__ void pair_slice(const RolloutDev<float>& p, long long
   auto fly = [&](const auto& oa, const auto& ob) {
     auto with_log = [&](auto& lg) {
       const Ground gr{a.ground_on, a.ground_z};
-      if constexpr (MC) rollout_run_pair<MODE, LAG>(d, c, acc, u, va, vb, v2, vo, ma, mb, tick0, n_ticks, a.inner_per_outer, oa, ob, lg, gr);
-      else rollout_run_pair<MODE, LAG>(d, c, acc, u, va, vb, p.vp, vo, ma, mb, tick0, n_ticks, a.inner_per_outer, oa, ob, lg, gr);
+      if constexpr (kSpecBody<MODE, std::decay_t<decltype(lg)>>) {
+        // speculative bodies: this thread's checkpoint slot after the staged boxes (launch_rollout sizes the area); made only here, so
+        // that the other bodies compile to the same code as before
+        const SpecSlot slot{(shared_boxes ? (24 * a.n_obs + 15) / 16 : 0) + (int)(threadIdx.x >> 5) * (32 * kSpecSlotVec4) + (int)(threadIdx.x & 31),
+                            spec_exact};
+        if constexpr (MC) rollout_run_pair<MODE, LAG>(d, c, acc, u, va, vb, v2, vo, ma, mb, tick0, n_ticks, a.inner_per_outer, oa, ob, lg, gr, slot);
+        else rollout_run_pair<MODE, LAG>(d, c, acc, u, va, vb, p.vp, vo, ma, mb, tick0, n_ticks, a.inner_per_outer, oa, ob, lg, gr, slot);
+      } else {
+        if constexpr (MC) rollout_run_pair<MODE, LAG>(d, c, acc, u, va, vb, v2, vo, ma, mb, tick0, n_ticks, a.inner_per_outer, oa, ob, lg, gr);
+        else rollout_run_pair<MODE, LAG>(d, c, acc, u, va, vb, p.vp, vo, ma, mb, tick0, n_ticks, a.inner_per_outer, oa, ob, lg, gr);
+      }
     };
     if constexpr (LOG == 3) {
       PairTrajLog lg;
@@ -581,7 +590,8 @@ __device__ __forceinline__ int ld_acquire_gpu(const int* p) {
 __device__ __forceinline__ void st_release_gpu(int* p, int v) { asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
 
 template <bool MC, int MODE, int LOG, bool LAG>
-__device__ __forceinline__ void sliced_body(const RolloutDev<float>& p, const SliceSched& sch, const LogTma* maps, const TableSetDev* tabs = nullptr) {
+__device__ __forceinline__ void sliced_body(const RolloutDev<float>& p, const SliceSched& sch, const LogTma* maps, const TableSetDev* tabs = nullptr,
+                                            int spec_exact = 0) {
   extern __shared__ __align__(128) float s_boxes[];
   __shared__ int s_item;
   stage_shared_boxes(p.a, s_boxes);
@@ -604,7 +614,7 @@ __device__ __forceinline__ void sliced_body(const RolloutDev<float>& p, const Sl
       const bool last = c == sch.n_chunks - 1;
       const int t0 = sch.begin(c);
       const int ticks = last ? p.a.n_ticks - t0 : sch.begin(c + 1) - t0;
-      pair_slice<LOG, MC, MODE, LAG>(p, j, ticks, c > 0 || p.a.resume != 0, !last || sch.final_carry != 0, last, t0, maps, c == 0, tabs);
+      pair_slice<LOG, MC, MODE, LAG>(p, j, ticks, c > 0 || p.a.resume != 0, !last || sch.final_carry != 0, last, t0, maps, c == 0, tabs, spec_exact);
     }
     __threadfence();
     __syncthreads();
@@ -612,9 +622,10 @@ __device__ __forceinline__ void sliced_body(const RolloutDev<float>& p, const Sl
   }
 }
 
+// spec_exact: development switch of the speculative bodies (uavb_dev_speculation), read by the metrics-only table bodies only
 template <bool MC, bool TABLE, bool LOG, bool LAG>
-__global__ void __maxnreg__(kRolloutPairRegs) rollout_sliced_kernel(const __grid_constant__ RolloutDev<float> p, const SliceSched sch) {
-  sliced_body<MC, TABLE ? kTargetShared : kTargetFly, LOG ? 1 : 0, LAG>(p, sch, nullptr);
+__global__ void __maxnreg__(kRolloutPairRegs) rollout_sliced_kernel(const __grid_constant__ RolloutDev<float> p, const SliceSched sch, int spec_exact) {
+  sliced_body<MC, TABLE ? kTargetShared : kTargetFly, LOG ? 1 : 0, LAG>(p, sch, nullptr, nullptr, spec_exact);
 }
 
 // One drone per thread at 128 registers, 16 one-warp CTAs per SM: the round-1 kernel, kept for metrics-only rollouts with PER-ROLLOUT
@@ -672,8 +683,8 @@ __global__ void __maxnreg__(kRolloutPairRegs) rollout_sliced_tma_kernel(const __
 // stores, the flown-path list, staged tensor stores.  `ts` lives in the kernel parameter space like `maps`.
 template <bool MC, bool LOG, bool LAG>
 __global__ void __maxnreg__(kRolloutPairRegs) rollout_sliced_tables_kernel(const __grid_constant__ RolloutDev<float> p, const SliceSched sch,
-                                                                            const __grid_constant__ TableSetDev ts) {
-  sliced_body<MC, kTargetPerRollout, LOG ? 1 : 0, LAG>(p, sch, nullptr, &ts);
+                                                                            const __grid_constant__ TableSetDev ts, int spec_exact) {
+  sliced_body<MC, kTargetPerRollout, LOG ? 1 : 0, LAG>(p, sch, nullptr, &ts, spec_exact);
 }
 template <bool MC, bool LAG>
 __global__ void __maxnreg__(kRolloutPairRegs) rollout_sliced_tables_traj_kernel(const __grid_constant__ RolloutDev<float> p, const SliceSched sch,
@@ -697,6 +708,25 @@ void launch_rollout_tables(bool mc, bool traj, int grid, size_t smem, cudaStream
                            const TableSetDev& ts);
 void launch_rollout_tables_log(bool mc, int grid, size_t smem, cudaStream_t st, const RolloutDev<float>& p, const SliceSched& sch,
                                const LogTma* maps, const TableSetDev& ts);
+// Development switch of the speculative bodies (rollout_pair.cuh, set by uavb_dev_speculation): fly every stretch exactly.
+extern int g_spec_exact;
+// Counting builds (UAVB_SPEC_COUNT): read (and zero) the stretch counters of one translation unit (8 words; zeros otherwise).
+cudaError_t spec_counts_sliced(unsigned long long* counts, bool reset);
+cudaError_t spec_counts_tables(unsigned long long* counts, bool reset);
+template <int TU> static cudaError_t spec_counts(unsigned long long* counts, bool reset) {
+#if UAVB_SPEC_COUNT
+  cudaError_t e = cudaMemcpyFromSymbol(counts, g_spec_count, sizeof(g_spec_count));
+  if (e == cudaSuccess && reset) {
+    const unsigned long long z[8] = {};
+    e = cudaMemcpyToSymbol(g_spec_count, z, sizeof(z));
+  }
+  return e;
+#else
+  (void)reset;
+  for (int k = 0; k < 8; ++k) counts[k] = 0;
+  return cudaSuccess;
+#endif
+}
 void launch_rollout_sliced_scalar(bool mc, int grid, size_t smem, cudaStream_t st, const RolloutDev<float>& p, const SliceSched& sch);
 void launch_rollout_f64(bool log, bool mc, int grid, size_t smem, cudaStream_t st, const RolloutDev<double>& p);
 

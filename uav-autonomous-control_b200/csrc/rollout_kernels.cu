@@ -9,6 +9,8 @@
 
 namespace uavb {
 
+int g_spec_exact = 0;
+
 // ---------------------------------------------------------------------------------------------
 // Set-point table of a shared mission.  Pass 1 (one thread per row): polynomial values and the row's own heading
 // (velocity direction where the horizontal speed reaches the threshold, NaN elsewhere).  Pass 2: every row takes the
@@ -223,6 +225,12 @@ template <class R> static int launch_rollout(const uavb_rollout_args* a, void* s
       }
       sch.n_tab = n; sch.n_chunks = n;
     }
+    // metrics-only shared-table / per-rollout-table bodies: the speculative stretches' checkpoints (rollout_pair.cuh), 160 B per thread
+    // after the staged boxes -- 5 KB per one-warp CTA, 8 CTAs per SM stay resident
+    if (!log && a->traj_out == nullptr && !scalar32 && (from_table || tabs) && UAVB_SPECULATE) {
+      smem = (smem + 15) / 16 * 16;
+      smem += sizeof(float4) * kSpecSlotVec4 * threads;
+    }
     const int pgrid = slots < grid ? slots : grid;
     // state log: through the TMA unit when the [samples x 13][B] log is a legal tensor (rows a multiple of 16 bytes, 16-byte aligned)
     LogTma maps;
@@ -332,6 +340,24 @@ extern "C" int uavb_rollout_targets_f64(const double* seg_coeffs, const int* seg
   UAVB_CUDA_OK(cudaGetLastError());
   target_heading_kernel<<<div_up(n_rows, 128), 128, 0, st>>>(raw, tstart, seg_yaw0, seg_rows, n_seg, out, n_rows);
   UAVB_CUDA_OK(cudaGetLastError());
+  return UAVB_OK;
+}
+
+// Development entry point, not part of uavb.h (tests/test_speculative_gpu.py, tools/spec_probe.py): force_exact = 1 flies every
+// stretch of the speculative kernels with the exact body in later launches, 0 restores speculation (< 0: unchanged);
+// counts (8 words, may be NULL) receives the stretch counters of a counting build (UAVB_SPEC_COUNT), summed over the kernels, and
+// reset = 1 zeroes them.
+extern "C" int uavb_dev_speculation(int force_exact, unsigned long long* counts, int reset) {
+  using namespace uavb;
+  if (force_exact >= 0) g_spec_exact = force_exact != 0;
+  if (!counts && !reset) return UAVB_OK;
+  int rc = require_device();
+  if (rc) return rc;
+  unsigned long long c0[8], c1[8];
+  UAVB_CUDA_OK(spec_counts_sliced(c0, reset != 0));
+  UAVB_CUDA_OK(spec_counts_tables(c1, reset != 0));
+  if (counts)
+    for (int k = 0; k < 8; ++k) counts[k] = c0[k] + c1[k];
   return UAVB_OK;
 }
 

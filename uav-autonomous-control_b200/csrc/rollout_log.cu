@@ -17,11 +17,11 @@ template <bool LAG> static void launch_tma(bool mc, bool table, int grid, size_t
 
 template <bool LAG> static void launch_lag(bool mc, bool table, int grid, size_t smem, cudaStream_t st, const RolloutDev<float>& p, const SliceSched& sch) {
   if (table) {
-    if (mc) rollout_sliced_kernel<true, true, true, LAG><<<grid, kRolloutThreadsLog, smem, st>>>(p, sch);
-    else rollout_sliced_kernel<false, true, true, LAG><<<grid, kRolloutThreadsLog, smem, st>>>(p, sch);
+    if (mc) rollout_sliced_kernel<true, true, true, LAG><<<grid, kRolloutThreadsLog, smem, st>>>(p, sch, 0);
+    else rollout_sliced_kernel<false, true, true, LAG><<<grid, kRolloutThreadsLog, smem, st>>>(p, sch, 0);
   } else {
-    if (mc) rollout_sliced_kernel<true, false, true, LAG><<<grid, kRolloutThreadsLog, smem, st>>>(p, sch);
-    else rollout_sliced_kernel<false, false, true, LAG><<<grid, kRolloutThreadsLog, smem, st>>>(p, sch);
+    if (mc) rollout_sliced_kernel<true, false, true, LAG><<<grid, kRolloutThreadsLog, smem, st>>>(p, sch, 0);
+    else rollout_sliced_kernel<false, false, true, LAG><<<grid, kRolloutThreadsLog, smem, st>>>(p, sch, 0);
   }
 }
 

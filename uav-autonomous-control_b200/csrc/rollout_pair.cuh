@@ -12,6 +12,8 @@
 #include "rollout_core.cuh"
 #include "tma.cuh"
 
+#include <type_traits>
+
 #ifndef UAVB_TICK_UNROLL
 #define UAVB_TICK_UNROLL 2
 #endif
@@ -160,6 +162,70 @@ enum : int { kTargetFly = 0, kTargetShared = 1, kTargetPerRollout = 2 };
 #endif
 constexpr int kTablesTickUnroll = UAVB_TABLES_TICK_UNROLL;
 
+// Speculative stretches (metrics-only bodies of the shared-table and per-rollout-table modes).  The exact tick carries two rare
+// paths -- the rotor-limit path and the large-rotation quaternion map -- and the branch around each keeps the next tick's head
+// from being scheduled against this tick's body.  A non-watching stretch therefore flies the branch-free inner_tick_pair_spec, with
+// the fields the tick writes checkpointed in shared memory first; when some lane of the warp would have taken a rare path, the warp
+// reloads the checkpoint and flies the same ticks with the exact body.  Without a rare path both bodies execute the same rounded
+// operations, so results are bit-identical either way.
+//   UAVB_SPECULATE    0 = always the exact body (the kernels of the previous release)
+//   UAVB_SPEC_HOLD    non-watching stretches flown with the exact body after a rollback (rare paths cluster in mission phases)
+//   UAVB_SPEC_UNROLL  ticks per iteration of the speculative loop
+#ifndef UAVB_SPECULATE
+#define UAVB_SPECULATE 1
+#endif
+#ifndef UAVB_SPEC_HOLD
+#define UAVB_SPEC_HOLD 4
+#endif
+#ifndef UAVB_SPEC_UNROLL
+#define UAVB_SPEC_UNROLL 2
+#endif
+constexpr int kSpecHold = UAVB_SPEC_HOLD;
+constexpr int kSpecUnroll = UAVB_SPEC_UNROLL;
+constexpr int kSpecSlotVec4 = 10;                            // 20 float2 fields of Drone2 = 10 x 16 bytes per thread
+template <int MODE, class LOG> constexpr bool kSpecBody = UAVB_SPECULATE && std::is_same<LOG, NoPairLog>::value && MODE != kTargetFly;
+
+// One thread's checkpoint in dynamic shared memory: 16-byte words k = 0..9 at s_spec[base + 32 k], base = the slot area (after the
+// staged boxes) + 320 words per warp + the lane -- a warp's store of one word is 512 contiguous bytes, conflict-free, and the
+// addresses are 32-bit shared-window offsets.
+extern __shared__ __align__(16) float4 s_spec[];
+struct SpecSlot {
+  int base;
+  int exact;               // development switch (uavb_dev_speculation): fly every stretch with the exact body
+  UAVB_DEV float4& w(int k) const { return s_spec[base + 32 * k]; }
+  UAVB_DEV void save(const Drone2& d) const {
+    w(0) = make_float4(d.dx.x, d.dx.y, d.dy.x, d.dy.y);
+    w(1) = make_float4(d.dz.x, d.dz.y, d.q0.x, d.q0.y);
+    w(2) = make_float4(d.q1.x, d.q1.y, d.q2.x, d.q2.y);
+    w(3) = make_float4(d.q3.x, d.q3.y, d.vx.x, d.vx.y);
+    w(4) = make_float4(d.vy.x, d.vy.y, d.vz.x, d.vz.y);
+    w(5) = make_float4(d.wx.x, d.wx.y, d.wy.x, d.wy.y);
+    w(6) = make_float4(d.wz.x, d.wz.y, d.om0.x, d.om0.y);
+    w(7) = make_float4(d.om1.x, d.om1.y, d.om2.x, d.om2.y);
+    w(8) = make_float4(d.om3.x, d.om3.y, d.zbx.x, d.zbx.y);
+    w(9) = make_float4(d.zby.x, d.zby.y, d.zbz.x, d.zbz.y);
+  }
+  UAVB_DEV void load(Drone2& d) const {
+    float4 t;
+    t = w(0); d.dx = make_float2(t.x, t.y); d.dy = make_float2(t.z, t.w);
+    t = w(1); d.dz = make_float2(t.x, t.y); d.q0 = make_float2(t.z, t.w);
+    t = w(2); d.q1 = make_float2(t.x, t.y); d.q2 = make_float2(t.z, t.w);
+    t = w(3); d.q3 = make_float2(t.x, t.y); d.vx = make_float2(t.z, t.w);
+    t = w(4); d.vy = make_float2(t.x, t.y); d.vz = make_float2(t.z, t.w);
+    t = w(5); d.wx = make_float2(t.x, t.y); d.wy = make_float2(t.z, t.w);
+    t = w(6); d.wz = make_float2(t.x, t.y); d.om0 = make_float2(t.z, t.w);
+    t = w(7); d.om1 = make_float2(t.x, t.y); d.om2 = make_float2(t.z, t.w);
+    t = w(8); d.om3 = make_float2(t.x, t.y); d.zbx = make_float2(t.z, t.w);
+    t = w(9); d.zby = make_float2(t.x, t.y); d.zbz = make_float2(t.z, t.w);
+  }
+};
+
+// Counting builds (UAVB_SPEC_COUNT, development only): per-warp counts of the stretches [watching, non-watching, speculated, rolled
+// back, some lane failed the sufficient rotor-limit test, some lane had a large rotation], one copy per translation unit.
+#if UAVB_SPEC_COUNT
+static __device__ unsigned long long g_spec_count[8];
+#endif
+
 // Set-points of the coming outer period and the position errors (set-point - position, fp64, rounded once): one table row
 // for both lanes of a shared mission, otherwise each lane's own cursor or table.
 template <int MODE> struct PairTarget;
@@ -271,10 +337,14 @@ template <int L, class OBST> UAVB_DEV void pair_hit(const Drone2& d, Accum<float
 template <int MODE, bool LAG, class VP2, class OBST, class LOG>
 UAVB_DEV void rollout_run_pair(Drone2& d, Cursor<float> (&c)[2], Accum<float> (&a)[2], const VehU<float>& u, const VehP<float>& va,
                                const VehP<float>& vb, const VP2& v2, const VehO2& vo, const MissionView& ma, const MissionView& mb, int tick0,
-                               int n_ticks, int freq, const OBST& oa, const OBST& ob, LOG& logger, const Ground gr = Ground{0, 0.0}) {
+                               int n_ticks, int freq, const OBST& oa, const OBST& ob, LOG& logger, const Ground gr = Ground{0, 0.0},
+                               const SpecSlot slot = SpecSlot{0, 0}) {
   int k = 0;
   V2 clear = make_float2(0.f, 0.f);                          // not part of the carry: every launch / slice measures first
   const V2 acc_max = make_float2(va.acc_max, vb.acc_max);
+  constexpr bool kSpec = kSpecBody<MODE, LOG>;
+  int hold = 0;                                              // non-watching stretches left to fly exactly (not carried: no effect on results)
+  if constexpr (kSpec) hold = slot.exact ? 0x7fffffff : 0;
   while (k < n_ticks) {
     if (c[0].phase == 0) {
       Target2<typename PairTarget<MODE>::T> t;
@@ -305,10 +375,44 @@ UAVB_DEV void rollout_run_pair(Drone2& d, Cursor<float> (&c)[2], Accum<float> (&
         logger.tick(d);
       }
     };
-    if (watch) {
-      stretch(BoolC<true>{});
+    if constexpr (kSpec) {
+      bool flown = false;
+      if (!watch && hold == 0) {                             // (warp-uniform)
+        slot.save(d);
+        unsigned rare = 0;
+#pragma unroll(LAG || !std::is_same<VP2, VehP2>::value ? kSpecUnroll : 1)
+        for (int j = 0; j < n; ++j) inner_tick_pair_spec<LAG>(d, u, v2, rare);
+        flown = !__any_sync(__activemask(), rare != 0);
+#if UAVB_SPEC_COUNT
+        const unsigned am = __activemask();
+        const bool lim = __any_sync(am, (rare >> kRareLimitBit) & 1u), rot = __any_sync(am, (rare >> kRareRotBit) & 1u);
+        if ((threadIdx.x & 31u) == (unsigned)(__ffs(am) - 1)) {
+          atomicAdd(&g_spec_count[2], 1ull);
+          if (!flown) atomicAdd(&g_spec_count[3], 1ull);
+          if (lim) atomicAdd(&g_spec_count[4], 1ull);
+          if (rot) atomicAdd(&g_spec_count[5], 1ull);
+        }
+#endif
+        if (!flown) {                                        // roll back: the same n ticks with the exact body
+          slot.load(d);
+          hold = kSpecHold + 1;
+        }
+      }
+      if (!watch && hold > 0) --hold;
+#if UAVB_SPEC_COUNT
+      if ((threadIdx.x & 31u) == (unsigned)(__ffs(__activemask()) - 1)) atomicAdd(&g_spec_count[watch ? 0 : 1], 1ull);
+#endif
+      if (watch) {
+        stretch(BoolC<true>{});
+      } else if (!flown) {
+        stretch(BoolC<false>{});
+      }
     } else {
-      stretch(BoolC<false>{});
+      if (watch) {
+        stretch(BoolC<true>{});
+      } else {
+        stretch(BoolC<false>{});
+      }
     }
     k += n;
     c[0].phase += n;

@@ -11,8 +11,8 @@ template <bool LAG> static void launch_lag(bool mc, int grid, size_t smem, cudaS
     if (mc) rollout_sliced_tables_tma_kernel<true, LAG><<<grid, kRolloutThreadsLog, smem, st>>>(p, sch, *maps, ts);
     else rollout_sliced_tables_tma_kernel<false, LAG><<<grid, kRolloutThreadsLog, smem, st>>>(p, sch, *maps, ts);
   } else {
-    if (mc) rollout_sliced_tables_kernel<true, true, LAG><<<grid, kRolloutThreadsLog, smem, st>>>(p, sch, ts);
-    else rollout_sliced_tables_kernel<false, true, LAG><<<grid, kRolloutThreadsLog, smem, st>>>(p, sch, ts);
+    if (mc) rollout_sliced_tables_kernel<true, true, LAG><<<grid, kRolloutThreadsLog, smem, st>>>(p, sch, ts, 0);
+    else rollout_sliced_tables_kernel<false, true, LAG><<<grid, kRolloutThreadsLog, smem, st>>>(p, sch, ts, 0);
   }
 }
 
