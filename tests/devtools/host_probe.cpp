@@ -62,7 +62,7 @@ template <class R> int run(const char* in, const char* outp) {
   std::vector<double> log;
   VecLog<R> lg{&log, 10, 10};
   NoObstacles no;
-  rollout_run<R, false>(d, c, a, u, v, m, 0, n_ticks, 10, lag, no, lg);
+  rollout_run<R>(d, c, a, u, v, m, 0, n_ticks, 10, lag, no, lg);
   FILE* g = fopen(outp, "wb");
   fwrite(log.data(), 8, log.size(), g);
   fclose(g);

@@ -222,8 +222,9 @@ template <bool NORM, bool LAG, class VP> UAVB_DEV void inner_tick_pair(Drone2& d
 // The speculative tick (rollout_run_pair): inner_tick_pair<false, LAG> without its two rare paths and without a branch.  It always
 // keeps the unclipped mixer outputs and the tan-form quaternion map; a lane where the exact tick would take the rotor-limit path
 // (failed sufficient test) or the large-rotation path (|w|^2 >= small_rot_wn2) sets its bit in `rare`, and its state is then wrong.
-// Where no bit is set the tick ran exactly the rounded operations of inner_tick_pair<false, LAG>.  (Kept as a copy rather than a
-// template switch of inner_tick_pair, so that the kernels that do not speculate compile to the same code as before.)
+// Where no bit is set the tick ran exactly the rounded operations of inner_tick_pair<false, LAG>, so the two must change together.
+// (A copy rather than a template switch of inner_tick_pair: as a switch, the same operations reach ptxas in another order and the
+// speculative kernels compile to different machine code.)
 // Bits of `rare`: one for both paths unless a counting build (UAVB_SPEC_COUNT, development only) tells them apart.
 #ifndef UAVB_SPEC_COUNT
 #define UAVB_SPEC_COUNT 0

@@ -160,9 +160,8 @@ template <class R> UAVB_HD void table_target(const TargetRow* rows, int row, Tar
 // again when the next stretch could use it up.  While clear > reach no box can be entered before the next check and the
 // per-tick inclusive point-in-AABB test (minimum_snap.py:352-357) is skipped for the stretch.  The flag and first-hit tick
 // are those of the per-tick test; only the work changes.
-// TABLE: the mission's set-points come from MissionView::trows (shared missions); otherwise they are evaluated on the fly.
-// A compile-time switch, so the table-driven instantiation carries none of the fp64 evaluation code or its registers.
-template <class R, bool TABLE, class OBST, class LOG>
+// Set-points are evaluated from the mission's splines (cursor_target).
+template <class R, class OBST, class LOG>
 UAVB_HD void rollout_run(Drone<R>& d, Cursor<R>& c, Accum<R>& a, const VehU<R>& u, const VehP<R>& v, const MissionView& m,
                          int tick0, int n_ticks, int freq, int lag, const OBST& obst, LOG& logger, const Ground gr = Ground{0, 0.0}) {
   typedef Math<R> M;
@@ -171,13 +170,8 @@ UAVB_HD void rollout_run(Drone<R>& d, Cursor<R>& c, Accum<R>& a, const VehU<R>& 
   while (k < n_ticks) {
     if (c.phase == 0) {
       Target<R> t;
-      if constexpr (TABLE) {
-        table_target<R>(m.trows, c.row, &t);
-        if (c.row + 1 < m.n_trows) ++c.row;                  // index clamp of main.py:61
-      } else {
-        cursor_target<R>(c, m, &t);
-        cursor_advance(&c.seg, &c.row, m);
-      }
+      cursor_target<R>(c, m, &t);
+      cursor_advance(&c.seg, &c.row, m);
       c.ex = (R)(t.x - d.px); c.ey = (R)(t.y - d.py); c.ez = (R)(t.z - d.pz);   // the position is folded here (d.dx = 0)
       outer_update<R>(d, u, v, t, c.ex, c.ey, c.ez);
     }

@@ -1,5 +1,7 @@
-// rollout_impl.cuh -- device side of K2, shared by the translation units that instantiate its kernels
-// (rollout_sliced.cu: metrics-only fp32; rollout_log.cu: fp32 with a state log; rollout_f64.cu: one-shot fp64 validation build).
+// rollout_impl.cuh -- device side of K2 and its launchers, shared by the translation units that instantiate its kernels
+// (two drones per thread, launch_pair: rollout_sliced.cu metrics only, rollout_log.cu state log, rollout_traj.cu flown-path list,
+// rollout_tables.cu / rollout_tables_log.cu per-rollout caller tables; rollout_scalar.cu: one drone per thread for per-rollout
+// missions; rollout_f64.cu: one-shot fp64 validation build).
 //
 // Each thread keeps its drone's 13-state, displacement accumulator, rotor speeds, controller integrator,
 // commands, table cursor and metric accumulators in registers for a whole slice of the mission (hundreds to
@@ -154,125 +156,6 @@ struct Carry {
   }
 };
 
-// One drone, one slice of its mission: `n_ticks` ticks starting from the carry block (from_carry) or from the start
-// pose; writes the carry block (to_carry) and / or the final outputs (finish).
-// MC: some per-rollout override (mass / inertia / gains / wind) is present; otherwise every vehicle constant is a
-// constant-bank operand.
-// `launch_tick0`: ticks of THIS launch that precede the slice (places the slice's samples in the state log).
-template <class R, bool LOG, bool MC, bool TABLE>
-__device__ __forceinline__ void drone_slice(const RolloutDev<R>& p, const float* s_boxes, long long i, int n_ticks, bool from_carry,
-                                            bool to_carry, bool finish, int launch_tick0 = 0) {
-  const uavb_rollout_args& a = p.a;
-  const long long B = a.B;
-  const bool shared_boxes = a.n_obs > 0 && a.aabb_set == nullptr;
-
-  // per-rollout constants
-  VehP<R> vloc;
-  if constexpr (MC) {
-    McValues mc;
-    mc_from_vehicle(mc, a.veh);
-    if (a.mc_mass) mc.mass = (double)a.mc_mass[i];
-    if (a.mc_inertia) { mc.inertia[0] = (double)a.mc_inertia[i]; mc.inertia[1] = (double)a.mc_inertia[B + i]; mc.inertia[2] = (double)a.mc_inertia[2 * B + i]; }
-    if (a.mc_gains) {
-#pragma unroll
-      for (int k = 0; k < UAVB_N_GAINS; ++k) mc.gains[k] = (double)a.mc_gains[k * B + i];
-    }
-    if (a.mc_wind) { mc.wind[0] = (double)a.mc_wind[i]; mc.wind[1] = (double)a.mc_wind[B + i]; mc.wind[2] = (double)a.mc_wind[2 * B + i]; }
-    make_vehp<R>(vloc, a.veh, mc);
-  }
-  const VehP<R>& v = MC ? vloc : p.vp;
-  const VehU<R>& u = p.u;
-
-  MissionView m;
-  m.coeffs = a.seg_coeffs; m.rows = a.seg_rows; m.table = a.seg_table; m.yaw0 = a.seg_yaw0;
-  m.seg_begin = a.mission_seg_begin ? a.mission_seg_begin[i] : 0;
-  m.seg_count = a.mission_seg_count ? a.mission_seg_count[i] : a.n_seg_shared;
-  m.dt_outer = a.dt_outer;
-  m.trows = a.mission_seg_begin ? nullptr : static_cast<const TargetRow*>(a.shared_targets);
-  m.n_trows = a.n_target_rows;
-  m.cache = nullptr; m.cache_stride = 0;
-  if (p.coeff_cache_offset >= 0) {             // on-the-fly evaluation: this thread's column of the CTA's coefficient staging area
-    extern __shared__ double s_dyn_f64[];
-    m.cache = s_dyn_f64 + p.coeff_cache_offset + threadIdx.x;
-    m.cache_stride = (int)blockDim.x;
-  }
-
-  Drone<R> d;
-  Cursor<R> c;
-  Accum<R> acc;
-  int tick0 = 0;
-  bool resumed = false;
-  if constexpr (sizeof(R) == 4) {
-    if (from_carry) {
-      Carry cb{a.carry + i, B};
-      cb.load(d, c, acc, u, &tick0);
-      resumed = true;
-    }
-  }
-  if (!resumed) {
-    const double* s = a.start + (size_t)a.start_stride * i;
-    drone_init<R>(d, u, s[0], s[1], s[2]);
-    cursor_init<R>(c);
-    accum_init<R>(acc);
-  }
-
-  auto fly = [&](const auto& obst) {
-    if constexpr (LOG) {
-      GlobalLog<R> lg;
-      lg.out = reinterpret_cast<R*>(a.log_out) + (size_t)(launch_tick0 / a.log_stride) * 13 * B + i;
-      lg.B = (unsigned)B; lg.stride = a.log_stride; lg.left = a.log_stride - launch_tick0 % a.log_stride;
-      rollout_run<R, TABLE>(d, c, acc, u, v, m, tick0, n_ticks, a.inner_per_outer, a.thrust_frame_lag, obst, lg, Ground{a.ground_on, a.ground_z});
-    } else {
-      NoLog lg;
-      rollout_run<R, TABLE>(d, c, acc, u, v, m, tick0, n_ticks, a.inner_per_outer, a.thrust_frame_lag, obst, lg, Ground{a.ground_on, a.ground_z});
-    }
-  };
-  // three call sites, not four: the flying code is inlined at each (a floor without boxes is the shared set with n = 0 -- the
-  // floor rides on the obstacle culling)
-  if (a.n_obs > 0 && !shared_boxes) {
-    fly(BoxesT<false>{a.aabbs + (size_t)a.aabb_set[i] * a.n_obs * 6, a.n_obs});
-  } else if (a.n_obs > 0 || a.ground_on) {
-    fly(BoxesT<true>{nullptr, a.n_obs});
-  } else {
-    fly(NoObstacles{});
-  }
-
-  if constexpr (sizeof(R) == 4) {
-    if (to_carry) {
-      Carry cb{a.carry + i, B};
-      cb.store(d, c, acc, tick0 + n_ticks);
-    }
-  }
-  if (!finish) return;
-  const double fx = d.px + (double)d.dx, fy = d.py + (double)d.dy, fz = d.pz + (double)d.dz;
-  if (a.state_out) {
-    R* o = reinterpret_cast<R*>(a.state_out) + i;
-    o[0 * B] = (R)fx; o[1 * B] = (R)fy; o[2 * B] = (R)fz;
-    if (!LOG && c.phase != 0) renormalise_q<R>(d);           // the reported state is unit even in the middle of an outer period
-    o[3 * B] = d.q0; o[4 * B] = d.q1; o[5 * B] = d.q2; o[6 * B] = d.q3;
-    o[7 * B] = d.vx; o[8 * B] = d.vy; o[9 * B] = d.vz;
-    o[10 * B] = d.wx; o[11 * B] = d.wy; o[12 * B] = d.wz;
-  }
-  if (a.metrics_out) {
-    R fd = R(0);
-    if (a.goal) {
-      const double* g = a.goal + (size_t)a.goal_stride * i;
-      const R ex = (R)(g[0] - fx), ey = (R)(g[1] - fy), ez = (R)(g[2] - fz);
-      fd = Math<R>::sqrt(ex * ex + ey * ey + ez * ez);
-    }
-    const R np = acc.periods > 0 ? R(1) / (R)acc.periods : R(0);
-    R* o = reinterpret_cast<R*>(a.metrics_out) + (size_t)i * UAVB_N_METRICS;
-    o[UAVB_M_FINAL_DIST] = fd;
-    o[UAVB_M_COLLISION] = (R)acc.collided;
-    o[UAVB_M_RMSE] = Math<R>::sqrt(acc.sum_e2 * np);
-    o[UAVB_M_MEAN_ERR] = acc.sum_e * np;
-    o[UAVB_M_MAX_ERR] = acc.max_e;
-    o[UAVB_M_STATUS] = (R)acc.status;
-    o[UAVB_M_FIRST_HIT] = (R)acc.first_hit;
-    o[UAVB_M_PERIODS] = (R)acc.periods;
-  }
-}
-
 // Per-rollout constants of drone i (Monte-Carlo overrides applied).
 template <class R> __device__ __forceinline__ void load_vehp(VehP<R>& v, const uavb_rollout_args& a, long long i) {
   const long long B = a.B;
@@ -314,8 +197,8 @@ __device__ __forceinline__ void vehp_cache_load(const float* cache, long long st
 #undef UAVB_LD
 }
 
-__device__ __forceinline__ void mission_view(MissionView& m, const RolloutDev<float>& p, long long i, int column, int columns) {
-  const uavb_rollout_args& a = p.a;
+// The mission of drone i; `column` of `columns`: its column of the CTA's coefficient staging area (RolloutDev::coeff_cache_offset).
+__device__ __forceinline__ void mission_view(MissionView& m, const uavb_rollout_args& a, int coeff_cache_offset, long long i, int column, int columns) {
   m.coeffs = a.seg_coeffs; m.rows = a.seg_rows; m.table = a.seg_table; m.yaw0 = a.seg_yaw0;
   m.seg_begin = a.mission_seg_begin ? a.mission_seg_begin[i] : 0;
   m.seg_count = a.mission_seg_count ? a.mission_seg_count[i] : a.n_seg_shared;
@@ -323,9 +206,9 @@ __device__ __forceinline__ void mission_view(MissionView& m, const RolloutDev<fl
   m.trows = a.mission_seg_begin ? nullptr : static_cast<const TargetRow*>(a.shared_targets);
   m.n_trows = a.n_target_rows;
   m.cache = nullptr; m.cache_stride = 0;
-  if (p.coeff_cache_offset >= 0) {             // on-the-fly evaluation: this drone's column of the CTA's coefficient staging area
+  if (coeff_cache_offset >= 0) {               // on-the-fly evaluation: this drone's column of the CTA's coefficient staging area
     extern __shared__ double s_dyn_f64[];
-    m.cache = s_dyn_f64 + p.coeff_cache_offset + column;
+    m.cache = s_dyn_f64 + coeff_cache_offset + column;
     m.cache_stride = columns;
   }
 }
@@ -350,37 +233,106 @@ __device__ __forceinline__ void table_view(MissionView& m, const TableSetDev& ts
   m.cache = nullptr; m.cache_stride = 0;
 }
 
-// Final outputs of one drone (state, metrics) -- shared by the pair path; same values as drone_slice's epilogue.
-__device__ __forceinline__ void write_outputs(const uavb_rollout_args& a, long long i, Drone<float>& d, const Cursor<float>& c,
-                                              const Accum<float>& acc, bool log) {
-  const long long B = a.B;
+// Final outputs of one drone (state, metrics).  B: a.B, passed in so that drone_slice's one load of it serves the whole slice.
+// log: the quaternion was renormalised in every tick (state-log bodies).
+template <class R> __device__ __forceinline__ void write_outputs(const uavb_rollout_args& a, long long B, long long i, Drone<R>& d, const Cursor<R>& c,
+                                                                const Accum<R>& acc, bool log) {
   const double fx = d.px + (double)d.dx, fy = d.py + (double)d.dy, fz = d.pz + (double)d.dz;
   if (a.state_out) {
-    float* o = reinterpret_cast<float*>(a.state_out) + i;
-    o[0 * B] = (float)fx; o[1 * B] = (float)fy; o[2 * B] = (float)fz;
-    if (!log && c.phase != 0) renormalise_q<float>(d);       // the reported state is unit even in the middle of an outer period
+    R* o = reinterpret_cast<R*>(a.state_out) + i;
+    o[0 * B] = (R)fx; o[1 * B] = (R)fy; o[2 * B] = (R)fz;
+    if (!log && c.phase != 0) renormalise_q<R>(d);           // the reported state is unit even in the middle of an outer period
     o[3 * B] = d.q0; o[4 * B] = d.q1; o[5 * B] = d.q2; o[6 * B] = d.q3;
     o[7 * B] = d.vx; o[8 * B] = d.vy; o[9 * B] = d.vz;
     o[10 * B] = d.wx; o[11 * B] = d.wy; o[12 * B] = d.wz;
   }
   if (a.metrics_out) {
-    float fd = 0.f;
+    R fd = R(0);
     if (a.goal) {
       const double* g = a.goal + (size_t)a.goal_stride * i;
-      const float ex = (float)(g[0] - fx), ey = (float)(g[1] - fy), ez = (float)(g[2] - fz);
-      fd = Math<float>::sqrt(ex * ex + ey * ey + ez * ez);
+      const R ex = (R)(g[0] - fx), ey = (R)(g[1] - fy), ez = (R)(g[2] - fz);
+      fd = Math<R>::sqrt(ex * ex + ey * ey + ez * ez);
     }
-    const float np = acc.periods > 0 ? 1.f / (float)acc.periods : 0.f;
-    float* o = reinterpret_cast<float*>(a.metrics_out) + (size_t)i * UAVB_N_METRICS;
+    const R np = acc.periods > 0 ? R(1) / (R)acc.periods : R(0);
+    R* o = reinterpret_cast<R*>(a.metrics_out) + (size_t)i * UAVB_N_METRICS;
     o[UAVB_M_FINAL_DIST] = fd;
-    o[UAVB_M_COLLISION] = (float)acc.collided;
-    o[UAVB_M_RMSE] = Math<float>::sqrt(acc.sum_e2 * np);
+    o[UAVB_M_COLLISION] = (R)acc.collided;
+    o[UAVB_M_RMSE] = Math<R>::sqrt(acc.sum_e2 * np);
     o[UAVB_M_MEAN_ERR] = acc.sum_e * np;
     o[UAVB_M_MAX_ERR] = acc.max_e;
-    o[UAVB_M_STATUS] = (float)acc.status;
-    o[UAVB_M_FIRST_HIT] = (float)acc.first_hit;
-    o[UAVB_M_PERIODS] = (float)acc.periods;
+    o[UAVB_M_STATUS] = (R)acc.status;
+    o[UAVB_M_FIRST_HIT] = (R)acc.first_hit;
+    o[UAVB_M_PERIODS] = (R)acc.periods;
   }
+}
+
+// One drone, one slice of its mission: `n_ticks` ticks starting from the carry block (from_carry) or from the start
+// pose; writes the carry block (to_carry) and / or the final outputs (finish).
+// MC: some per-rollout override (mass / inertia / gains / wind) is present; otherwise every vehicle constant is a
+// constant-bank operand.
+// `launch_tick0`: ticks of THIS launch that precede the slice (places the slice's samples in the state log).
+template <class R, bool LOG, bool MC>
+__device__ __forceinline__ void drone_slice(const RolloutDev<R>& p, long long i, int n_ticks, bool from_carry, bool to_carry, bool finish,
+                                            int launch_tick0 = 0) {
+  const uavb_rollout_args& a = p.a;
+  const long long B = a.B;
+  const bool shared_boxes = a.n_obs > 0 && a.aabb_set == nullptr;
+
+  VehP<R> vloc;
+  if constexpr (MC) load_vehp<R>(vloc, a, i);
+  const VehP<R>& v = MC ? vloc : p.vp;
+  const VehU<R>& u = p.u;
+
+  MissionView m;
+  mission_view(m, a, p.coeff_cache_offset, i, threadIdx.x, blockDim.x);
+
+  Drone<R> d;
+  Cursor<R> c;
+  Accum<R> acc;
+  int tick0 = 0;
+  bool resumed = false;
+  if constexpr (sizeof(R) == 4) {
+    if (from_carry) {
+      Carry cb{a.carry + i, B};
+      cb.load(d, c, acc, u, &tick0);
+      resumed = true;
+    }
+  }
+  if (!resumed) {
+    const double* s = a.start + (size_t)a.start_stride * i;
+    drone_init<R>(d, u, s[0], s[1], s[2]);
+    cursor_init<R>(c);
+    accum_init<R>(acc);
+  }
+
+  auto fly = [&](const auto& obst) {
+    if constexpr (LOG) {
+      GlobalLog<R> lg;
+      lg.out = reinterpret_cast<R*>(a.log_out) + (size_t)(launch_tick0 / a.log_stride) * 13 * B + i;
+      lg.B = (unsigned)B; lg.stride = a.log_stride; lg.left = a.log_stride - launch_tick0 % a.log_stride;
+      rollout_run<R>(d, c, acc, u, v, m, tick0, n_ticks, a.inner_per_outer, a.thrust_frame_lag, obst, lg, Ground{a.ground_on, a.ground_z});
+    } else {
+      NoLog lg;
+      rollout_run<R>(d, c, acc, u, v, m, tick0, n_ticks, a.inner_per_outer, a.thrust_frame_lag, obst, lg, Ground{a.ground_on, a.ground_z});
+    }
+  };
+  // three call sites, not four: the flying code is inlined at each (a floor without boxes is the shared set with n = 0 -- the
+  // floor rides on the obstacle culling)
+  if (a.n_obs > 0 && !shared_boxes) {
+    fly(BoxesT<false>{a.aabbs + (size_t)a.aabb_set[i] * a.n_obs * 6, a.n_obs});
+  } else if (a.n_obs > 0 || a.ground_on) {
+    fly(BoxesT<true>{nullptr, a.n_obs});
+  } else {
+    fly(NoObstacles{});
+  }
+
+  if constexpr (sizeof(R) == 4) {
+    if (to_carry) {
+      Carry cb{a.carry + i, B};
+      cb.store(d, c, acc, tick0 + n_ticks);
+    }
+  }
+  if (finish) write_outputs(a, B, i, d, c, acc, LOG);
 }
 
 // One PAIR of drones (2j, 2j+1), one slice of their mission: the production fp32 path (rollout_pair.cuh).  Arguments as
@@ -423,8 +375,8 @@ __device__ __forceinline__ void pair_slice(const RolloutDev<float>& p, long long
     table_view(ma, *tabs, i0);
     table_view(mb, *tabs, i1);
   } else {
-    mission_view(ma, p, i0, 2 * (int)threadIdx.x, 2 * (int)blockDim.x);
-    mission_view(mb, p, i1, 2 * (int)threadIdx.x + 1, 2 * (int)blockDim.x);
+    mission_view(ma, a, p.coeff_cache_offset, i0, 2 * (int)threadIdx.x, 2 * (int)blockDim.x);
+    mission_view(mb, a, p.coeff_cache_offset, i1, 2 * (int)threadIdx.x + 1, 2 * (int)blockDim.x);
   }
 
   Drone2 d;
@@ -518,11 +470,11 @@ __device__ __forceinline__ void pair_slice(const RolloutDev<float>& p, long long
   Drone<float> s;
   get_lane<0>(d, s);
   if (to_carry) Carry{a.carry + i0, B}.store(s, c[0], acc[0], tick0 + n_ticks);
-  if (finish) write_outputs(a, i0, s, c[0], acc[0], kStateLog);
+  if (finish) write_outputs(a, a.B, i0, s, c[0], acc[0], kStateLog);
   if (second) {
     get_lane<1>(d, s);
     if (to_carry) Carry{a.carry + i1, B}.store(s, c[1], acc[1], tick0 + n_ticks);
-    if (finish) write_outputs(a, i1, s, c[1], acc[1], kStateLog);
+    if (finish) write_outputs(a, a.B, i1, s, c[1], acc[1], kStateLog);
   }
   if constexpr (LOG == 3) {
     if (to_carry) {
@@ -554,13 +506,7 @@ __global__ void __maxnreg__(kRolloutRegs) rollout_kernel(const __grid_constant__
   stage_shared_boxes(p.a, s_boxes);
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= p.a.B) return;
-  if constexpr (sizeof(R) == 4) {
-    if (p.a.shared_targets != nullptr && p.a.mission_seg_begin == nullptr) {
-      drone_slice<R, LOG, MC, true>(p, s_boxes, i, p.a.n_ticks, p.a.resume != 0, p.a.carry != nullptr, true);
-      return;
-    }
-  }
-  drone_slice<R, LOG, MC, false>(p, s_boxes, i, p.a.n_ticks, p.a.resume != 0, p.a.carry != nullptr, true);   // fp64: always on the fly
+  drone_slice<R, LOG, MC>(p, i, p.a.n_ticks, p.a.resume != 0, p.a.carry != nullptr, true);
 }
 
 // Time-sliced persistent launch (every fp32 rollout, with or without a state log).  When the batch needs between one and a few waves of
@@ -589,12 +535,11 @@ __device__ __forceinline__ int ld_acquire_gpu(const int* p) {
 }
 __device__ __forceinline__ void st_release_gpu(int* p, int v) { asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
 
-template <bool MC, int MODE, int LOG, bool LAG>
-__device__ __forceinline__ void sliced_body(const RolloutDev<float>& p, const SliceSched& sch, const LogTma* maps, const TableSetDev* tabs = nullptr,
-                                            int spec_exact = 0) {
-  extern __shared__ __align__(128) float s_boxes[];
+// The work-item loop of a persistent launch.  A thread flies PER drones (1: drone k, 2: the pair 2k, 2k+1) of its CTA's work group; for
+// every (chunk, group) item the CTA pulls it runs item(k, chunk, t0, ticks, last) -- `ticks` ticks from launch tick t0, `last`: the final
+// slice -- once the group's previous slice has completed, and publishes the item's completion.
+template <int PER, class F> __device__ __forceinline__ void slice_items(const uavb_rollout_args& a, const SliceSched& sch, F&& item) {
   __shared__ int s_item;
-  stage_shared_boxes(p.a, s_boxes);
   const int n_items = sch.n_groups * sch.n_chunks;
   for (;;) {
     if (threadIdx.x == 0) {
@@ -609,17 +554,27 @@ __device__ __forceinline__ void sliced_body(const RolloutDev<float>& p, const Sl
     const int it = s_item;
     if (it >= n_items) return;
     const int c = it / sch.n_groups, g = it - c * sch.n_groups;
-    const long long j = (long long)g * blockDim.x + threadIdx.x;        // pair index: drones 2j, 2j+1
-    if (2 * j < p.a.B) {
+    const long long k = (long long)g * blockDim.x + threadIdx.x;
+    if (PER * k < a.B) {
       const bool last = c == sch.n_chunks - 1;
       const int t0 = sch.begin(c);
-      const int ticks = last ? p.a.n_ticks - t0 : sch.begin(c + 1) - t0;
-      pair_slice<LOG, MC, MODE, LAG>(p, j, ticks, c > 0 || p.a.resume != 0, !last || sch.final_carry != 0, last, t0, maps, c == 0, tabs, spec_exact);
+      const int ticks = last ? a.n_ticks - t0 : sch.begin(c + 1) - t0;
+      item(k, c, t0, ticks, last);
     }
     __threadfence();
     __syncthreads();
     if (threadIdx.x == 0) st_release_gpu(sch.done + g, c + 1);
   }
+}
+
+template <bool MC, int MODE, int LOG, bool LAG>
+__device__ __forceinline__ void sliced_body(const RolloutDev<float>& p, const SliceSched& sch, const LogTma* maps, const TableSetDev* tabs = nullptr,
+                                            int spec_exact = 0) {
+  extern __shared__ __align__(128) float s_boxes[];
+  stage_shared_boxes(p.a, s_boxes);
+  slice_items<2>(p.a, sch, [&](long long j, int c, int t0, int ticks, bool last) {
+    pair_slice<LOG, MC, MODE, LAG>(p, j, ticks, c > 0 || p.a.resume != 0, !last || sch.final_carry != 0, last, t0, maps, c == 0, tabs, spec_exact);
+  });
 }
 
 // spec_exact: development switch of the speculative bodies (uavb_dev_speculation), read by the metrics-only table bodies only
@@ -637,33 +592,10 @@ constexpr int kScalarCtasPerSm = 16;
 template <bool MC>
 __global__ void __maxnreg__(kRolloutRegs) rollout_sliced_scalar_kernel(const __grid_constant__ RolloutDev<float> p, const SliceSched sch) {
   extern __shared__ __align__(128) float s_boxes[];
-  __shared__ int s_item;
   stage_shared_boxes(p.a, s_boxes);
-  const int n_items = sch.n_groups * sch.n_chunks;
-  for (;;) {
-    if (threadIdx.x == 0) {
-      const int it = atomicAdd(sch.counter, 1);
-      if (it < n_items) {
-        const int c = it / sch.n_groups, g = it - c * sch.n_groups;
-        while (ld_acquire_gpu(sch.done + g) < c) __nanosleep(200);
-      }
-      s_item = it;
-    }
-    __syncthreads();
-    const int it = s_item;
-    if (it >= n_items) return;
-    const int c = it / sch.n_groups, g = it - c * sch.n_groups;
-    const long long i = (long long)g * blockDim.x + threadIdx.x;
-    if (i < p.a.B) {
-      const bool last = c == sch.n_chunks - 1;
-      const int t0 = sch.begin(c);
-      const int ticks = last ? p.a.n_ticks - t0 : sch.begin(c + 1) - t0;
-      drone_slice<float, false, MC, false>(p, s_boxes, i, ticks, c > 0 || p.a.resume != 0, !last || sch.final_carry != 0, last, t0);
-    }
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) st_release_gpu(sch.done + g, c + 1);
-  }
+  slice_items<1>(p.a, sch, [&](long long i, int c, int t0, int ticks, bool last) {
+    drone_slice<float, false, MC>(p, i, ticks, c > 0 || p.a.resume != 0, !last || sch.final_carry != 0, last, t0);
+  });
 }
 
 // Metrics + the gated position list of the viewer (PairTrajLog); one-warp CTAs like the metrics-only kernel.
@@ -698,16 +630,6 @@ __global__ void __maxnreg__(kRolloutPairRegs) rollout_sliced_tables_tma_kernel(c
 }
 
 
-// Host-side launchers, one per translation unit (kernel templates are instantiated where they are launched).
-void launch_rollout_sliced(bool mc, bool table, int grid, size_t smem, cudaStream_t st, const RolloutDev<float>& p, const SliceSched& sch);
-void launch_rollout_sliced_log(bool mc, bool table, int grid, size_t smem, cudaStream_t st, const RolloutDev<float>& p, const SliceSched& sch,
-                               const LogTma* maps);      // maps != nullptr: staged tensor stores
-void launch_rollout_sliced_traj(bool mc, bool table, int grid, size_t smem, cudaStream_t st, const RolloutDev<float>& p, const SliceSched& sch);
-// per-rollout caller tables (rollout_tables.cu: metrics only / flown-path list; rollout_tables_log.cu: state log, maps as above)
-void launch_rollout_tables(bool mc, bool traj, int grid, size_t smem, cudaStream_t st, const RolloutDev<float>& p, const SliceSched& sch,
-                           const TableSetDev& ts);
-void launch_rollout_tables_log(bool mc, int grid, size_t smem, cudaStream_t st, const RolloutDev<float>& p, const SliceSched& sch,
-                               const LogTma* maps, const TableSetDev& ts);
 // Development switch of the speculative bodies (rollout_pair.cuh, set by uavb_dev_speculation): fly every stretch exactly.
 extern int g_spec_exact;
 // Counting builds (UAVB_SPEC_COUNT): read (and zero) the stretch counters of one translation unit (8 words; zeros otherwise).
@@ -727,6 +649,42 @@ template <int TU> static cudaError_t spec_counts(unsigned long long* counts, boo
   return cudaSuccess;
 #endif
 }
+
+// Launch of a pair kernel: MODE (kTargetFly / kTargetShared / kTargetPerRollout, `ts` required for the last) and LOG (as pair_slice;
+// 2 requires `maps`) pick the kernel family and its CTA shape, mc and lag its instantiation.  Each (MODE, LOG) is instantiated by the
+// translation unit that compiles its kernels (UAVB_LAUNCH_PAIR below), so that the units compile in parallel.
+template <int MODE, int LOG>
+void launch_pair(bool mc, bool lag, int grid, size_t smem, cudaStream_t st, const RolloutDev<float>& p, const SliceSched& sch, const LogTma* maps,
+                 const TableSetDev* ts) {
+  constexpr int threads = (LOG == 1 || LOG == 2) ? kRolloutThreadsLog : kRolloutThreads;
+  auto go = [&](auto mc_c, auto lag_c) {
+    constexpr bool MC = decltype(mc_c)::value, LAG = decltype(lag_c)::value;
+    if constexpr (MODE == kTargetPerRollout) {
+      if constexpr (LOG == 3) rollout_sliced_tables_traj_kernel<MC, LAG><<<grid, threads, smem, st>>>(p, sch, *ts);
+      else if constexpr (LOG == 2) rollout_sliced_tables_tma_kernel<MC, LAG><<<grid, threads, smem, st>>>(p, sch, *maps, *ts);
+      else rollout_sliced_tables_kernel<MC, LOG == 1, LAG><<<grid, threads, smem, st>>>(p, sch, *ts, g_spec_exact);
+    } else {
+      constexpr bool TABLE = MODE == kTargetShared;
+      if constexpr (LOG == 3) rollout_sliced_traj_kernel<MC, TABLE, LAG><<<grid, threads, smem, st>>>(p, sch);
+      else if constexpr (LOG == 2) rollout_sliced_tma_kernel<MC, TABLE, LAG><<<grid, threads, smem, st>>>(p, sch, *maps);
+      else rollout_sliced_kernel<MC, TABLE, LOG == 1, LAG><<<grid, threads, smem, st>>>(p, sch, g_spec_exact);
+    }
+  };
+  if (mc) {
+    if (lag) go(BoolC<true>{}, BoolC<true>{}); else go(BoolC<true>{}, BoolC<false>{});
+  } else {
+    if (lag) go(BoolC<false>{}, BoolC<true>{}); else go(BoolC<false>{}, BoolC<false>{});
+  }
+}
+#define UAVB_LAUNCH_PAIR(MODE, LOG)                                                                                                  \
+  template void launch_pair<MODE, LOG>(bool, bool, int, size_t, cudaStream_t, const RolloutDev<float>&, const SliceSched&, const LogTma*, \
+                                       const TableSetDev*)
+extern UAVB_LAUNCH_PAIR(kTargetFly, 0); extern UAVB_LAUNCH_PAIR(kTargetFly, 1); extern UAVB_LAUNCH_PAIR(kTargetFly, 2); extern UAVB_LAUNCH_PAIR(kTargetFly, 3);
+extern UAVB_LAUNCH_PAIR(kTargetShared, 0); extern UAVB_LAUNCH_PAIR(kTargetShared, 1); extern UAVB_LAUNCH_PAIR(kTargetShared, 2);
+extern UAVB_LAUNCH_PAIR(kTargetShared, 3);
+extern UAVB_LAUNCH_PAIR(kTargetPerRollout, 0); extern UAVB_LAUNCH_PAIR(kTargetPerRollout, 1); extern UAVB_LAUNCH_PAIR(kTargetPerRollout, 2);
+extern UAVB_LAUNCH_PAIR(kTargetPerRollout, 3);
+
 void launch_rollout_sliced_scalar(bool mc, int grid, size_t smem, cudaStream_t st, const RolloutDev<float>& p, const SliceSched& sch);
 void launch_rollout_f64(bool log, bool mc, int grid, size_t smem, cudaStream_t st, const RolloutDev<double>& p);
 

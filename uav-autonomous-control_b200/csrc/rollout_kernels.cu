@@ -1,6 +1,7 @@
 // rollout_kernels.cu -- K2 host side: argument checks, launch policy (time slicing, scratch), the set-point table of a
-// shared mission, and the C entry points.  The device code lives in rollout_impl.cuh and is instantiated in
-// rollout_sliced.cu / rollout_log.cu / rollout_f64.cu.
+// shared mission, and the C entry points.  The device code lives in rollout_impl.cuh; its kernels are instantiated, with their
+// launchers, in rollout_sliced.cu / rollout_log.cu / rollout_traj.cu / rollout_tables.cu / rollout_tables_log.cu (two drones per
+// thread), rollout_scalar.cu (one drone per thread) and rollout_f64.cu (fp64 validation build).
 #ifdef UAVB_DEV
 #include <stdlib.h>
 #endif
@@ -249,12 +250,19 @@ template <class R> static int launch_rollout(const uavb_rollout_args* a, void* s
         smem += sizeof(float) * kLogTmaWarpFloats * (kRolloutThreadsLog / 32);
       }
     }
-    if (tabs && log) launch_rollout_tables_log(mc_any, pgrid, smem, st, *reinterpret_cast<RolloutDev<float>*>(&p), sch, tma_log ? &maps : nullptr, *tabs);
-    else if (tabs) launch_rollout_tables(mc_any, a->traj_out != nullptr, pgrid, smem, st, *reinterpret_cast<RolloutDev<float>*>(&p), sch, *tabs);
-    else if (log) launch_rollout_sliced_log(mc_any, from_table, pgrid, smem, st, *reinterpret_cast<RolloutDev<float>*>(&p), sch, tma_log ? &maps : nullptr);
-    else if (scalar32) launch_rollout_sliced_scalar(mc_any, pgrid, smem, st, *reinterpret_cast<RolloutDev<float>*>(&p), sch);
-    else if (a->traj_out) launch_rollout_sliced_traj(mc_any, from_table, pgrid, smem, st, *reinterpret_cast<RolloutDev<float>*>(&p), sch);
-    else launch_rollout_sliced(mc_any, from_table, pgrid, smem, st, *reinterpret_cast<RolloutDev<float>*>(&p), sch);
+    const RolloutDev<float>& p32 = *reinterpret_cast<RolloutDev<float>*>(&p);
+    if (scalar32) {
+      launch_rollout_sliced_scalar(mc_any, pgrid, smem, st, p32, sch);
+    } else {
+      typedef void (*PairLaunch)(bool, bool, int, size_t, cudaStream_t, const RolloutDev<float>&, const SliceSched&, const LogTma*, const TableSetDev*);
+      static constexpr PairLaunch kPairLaunch[3][4] = {
+          {launch_pair<kTargetFly, 0>, launch_pair<kTargetFly, 1>, launch_pair<kTargetFly, 2>, launch_pair<kTargetFly, 3>},
+          {launch_pair<kTargetShared, 0>, launch_pair<kTargetShared, 1>, launch_pair<kTargetShared, 2>, launch_pair<kTargetShared, 3>},
+          {launch_pair<kTargetPerRollout, 0>, launch_pair<kTargetPerRollout, 1>, launch_pair<kTargetPerRollout, 2>, launch_pair<kTargetPerRollout, 3>}};
+      const int mode = tabs ? kTargetPerRollout : from_table ? kTargetShared : kTargetFly;
+      const int log_kind = log ? (tma_log ? 2 : 1) : a->traj_out ? 3 : 0;           // pair_slice's LOG
+      kPairLaunch[mode][log_kind](mc_any, a->thrust_frame_lag != 0, pgrid, smem, st, p32, sch, tma_log ? &maps : nullptr, tabs);
+    }
   }
   UAVB_CUDA_OK(cudaGetLastError());
   return UAVB_OK;

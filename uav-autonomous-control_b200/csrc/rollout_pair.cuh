@@ -246,6 +246,15 @@ template <> struct PairTarget<kTargetShared> {
     ez = make_float2((float)(t.z - d.pz[0]), (float)(t.z - d.pz[1]));
   }
 };
+// Zip the set-points of the two lanes and form their position errors.
+UAVB_DEV void zip_targets(const Drone2& d, const Target<float>& ta, const Target<float>& tb, Target2<V2>& t2, V2& ex, V2& ey, V2& ez) {
+  t2.vx = make_float2(ta.vx, tb.vx); t2.vy = make_float2(ta.vy, tb.vy); t2.vz = make_float2(ta.vz, tb.vz);
+  t2.ax = make_float2(ta.ax, tb.ax); t2.ay = make_float2(ta.ay, tb.ay); t2.az = make_float2(ta.az, tb.az);
+  t2.yc = make_float2(ta.yc, tb.yc); t2.ys = make_float2(ta.ys, tb.ys);
+  ex = make_float2((float)(ta.x - d.px[0]), (float)(tb.x - d.px[1]));
+  ey = make_float2((float)(ta.y - d.py[0]), (float)(tb.y - d.py[1]));
+  ez = make_float2((float)(ta.z - d.pz[0]), (float)(tb.z - d.pz[1]));
+}
 template <> struct PairTarget<kTargetFly> {
   typedef V2 T;
   static UAVB_DEV void fetch(const Drone2& d, Cursor<float> (&c)[2], const MissionView& ma, const MissionView& mb, Target2<V2>& t2, V2& ex, V2& ey, V2& ez) {
@@ -254,12 +263,7 @@ template <> struct PairTarget<kTargetFly> {
     cursor_advance(&c[0].seg, &c[0].row, ma);
     cursor_target<float>(c[1], mb, &tb);
     cursor_advance(&c[1].seg, &c[1].row, mb);
-    t2.vx = make_float2(ta.vx, tb.vx); t2.vy = make_float2(ta.vy, tb.vy); t2.vz = make_float2(ta.vz, tb.vz);
-    t2.ax = make_float2(ta.ax, tb.ax); t2.ay = make_float2(ta.ay, tb.ay); t2.az = make_float2(ta.az, tb.az);
-    t2.yc = make_float2(ta.yc, tb.yc); t2.ys = make_float2(ta.ys, tb.ys);
-    ex = make_float2((float)(ta.x - d.px[0]), (float)(tb.x - d.px[1]));
-    ey = make_float2((float)(ta.y - d.py[0]), (float)(tb.y - d.py[1]));
-    ez = make_float2((float)(ta.z - d.pz[0]), (float)(tb.z - d.pz[1]));
+    zip_targets(d, ta, tb, t2, ex, ey, ez);
   }
 };
 template <> struct PairTarget<kTargetPerRollout> {
@@ -278,12 +282,7 @@ template <> struct PairTarget<kTargetPerRollout> {
     asm volatile("prefetch.global.L1 [%0];" ::"l"(nb));
     asm volatile("prefetch.global.L1 [%0];" ::"l"(nb + sizeof(TargetRow) - 4));
 #endif
-    t2.vx = make_float2(ta.vx, tb.vx); t2.vy = make_float2(ta.vy, tb.vy); t2.vz = make_float2(ta.vz, tb.vz);
-    t2.ax = make_float2(ta.ax, tb.ax); t2.ay = make_float2(ta.ay, tb.ay); t2.az = make_float2(ta.az, tb.az);
-    t2.yc = make_float2(ta.yc, tb.yc); t2.ys = make_float2(ta.ys, tb.ys);
-    ex = make_float2((float)(ta.x - d.px[0]), (float)(tb.x - d.px[1]));
-    ey = make_float2((float)(ta.y - d.py[0]), (float)(tb.y - d.py[1]));
-    ez = make_float2((float)(ta.z - d.pz[0]), (float)(tb.z - d.pz[1]));
+    zip_targets(d, ta, tb, t2, ex, ey, ez);
   }
 };
 

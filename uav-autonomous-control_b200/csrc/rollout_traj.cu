@@ -4,19 +4,7 @@
 
 namespace uavb {
 
-template <bool LAG> static void launch_lag(bool mc, bool table, int grid, size_t smem, cudaStream_t st, const RolloutDev<float>& p, const SliceSched& sch) {
-  if (table) {
-    if (mc) rollout_sliced_traj_kernel<true, true, LAG><<<grid, kRolloutThreads, smem, st>>>(p, sch);
-    else rollout_sliced_traj_kernel<false, true, LAG><<<grid, kRolloutThreads, smem, st>>>(p, sch);
-  } else {
-    if (mc) rollout_sliced_traj_kernel<true, false, LAG><<<grid, kRolloutThreads, smem, st>>>(p, sch);
-    else rollout_sliced_traj_kernel<false, false, LAG><<<grid, kRolloutThreads, smem, st>>>(p, sch);
-  }
-}
-
-void launch_rollout_sliced_traj(bool mc, bool table, int grid, size_t smem, cudaStream_t st, const RolloutDev<float>& p, const SliceSched& sch) {
-  if (p.a.thrust_frame_lag) launch_lag<true>(mc, table, grid, smem, st, p, sch);
-  else launch_lag<false>(mc, table, grid, smem, st, p, sch);
-}
+UAVB_LAUNCH_PAIR(kTargetFly, 3);
+UAVB_LAUNCH_PAIR(kTargetShared, 3);
 
 }  // namespace uavb
