@@ -2,9 +2,12 @@
 // sampled-point AABB test of the correction loop.  All fp64, sm_100a.
 //
 // K1 is one thread per mission: ~2.5 k fp64 flops against 928 B of HBM traffic for S = 4
-// (SURVEY 8(d)), i.e. HBM-bound.  The per-mission output (8 S x 3 doubles, contiguous) is staged in
-// shared memory and leaves the CTA as one contiguous tile so every 32-byte sector is written whole.
-#include <stdlib.h>
+// (SURVEY 8(d)), i.e. HBM-bound.  For S <= 8 the per-mission output (8 S x 3 doubles, contiguous) is staged in
+// shared memory one or two splines at a time and leaves the CTA as whole 32-byte sectors:
+//   minsnap_solve_kernel<MAXS, kStageCopy1 | kStageCopy2>  by a copy loop over the CTA's threads (any output alignment);
+//   minsnap_solve_kernel<MAXS, kStageTma>                  by 2-D tensor stores (16-byte aligned output);
+//   minsnap_solve_stream_kernel                            the same stores from a persistent grid that bulk-loads its inputs (S = 4).
+// S > 8 stores straight from registers (kDirect), as does the ragged-S kernel of the correction loop.
 #include <mutex>
 
 #include "minsnap_core.cuh"
@@ -14,25 +17,51 @@
 
 namespace uavb {
 
-constexpr int kSolveThreads = 64;
+constexpr int kSolveThreads = 64;                          // missions per CTA (per tile of the streaming kernel)
+constexpr int kTmaSubTileBytes = kSolveThreads * 128;     // 64 rows x 16 doubles
+
+// K1's tensor-store staging: the 64 x 48-double tile of two splines leaves the CTA as three 2-D tensor stores
+// (cp.async.bulk.tensor.2d, boxes of 64 missions x 16 doubles over the [B][24 S] coefficient matrix) issued by one thread; it is
+// staged in the 128-byte swizzle the tensor map declares (16-byte chunk c of row r at chunk c ^ (r & 7)), and rows past the end of
+// the batch and the unused half of an odd last flush are clipped by the map.  NT staging tiles: splines 2k and 2k+1 are staged in
+// tile k % NT.  With one tile, the flush waits until the store has read it; with two, it waits for the store that read the OTHER
+// tile (a whole tile ago), and the kernel waits for the last stores itself before its shared memory goes.
+template <int NT>
+struct SwizzledTiles {
+  char* tiles;                                            // 1024-byte aligned (the swizzle period), NT x 3 sub-tiles
+  char* row;
+  unsigned sw;
+  __device__ __forceinline__ explicit SwizzledTiles(char* t) : tiles(t), row(t + threadIdx.x * 128), sw((threadIdx.x & 7u) << 4) {}
+  __device__ __forceinline__ void store(int seg, int j, int ax, double val) const {
+    const int off = (seg & 1) * 24 + j * 3 + ax, q = off >> 4, d = off & 15, tile = (seg >> 1) % NT;   // sub-tile, double within the 128-byte row
+    *reinterpret_cast<double*>(row + (tile * 3 + q) * kTmaSubTileBytes + ((((unsigned)d >> 1) << 4) ^ sw) + (d & 1) * 8) = val;
+  }
+  __device__ __forceinline__ void flush(const CUtensorMap* tmap, int seg, int S, long long base) const {
+    const bool last = seg == S - 1;
+    if (!(seg & 1) && !last) return;                      // uniform: S is the same for the whole launch
+    const int first = (seg & 1) ? seg - 1 : seg, n_sub = (seg & 1) ? 3 : 2, tile = (seg >> 1) % NT;   // a lone last spline fills 24 of the 48 columns
+    fence_proxy_async_smem();
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      for (int q = 0; q < n_sub; ++q) tensor_store_2d(tmap, first * 24 + q * 16, (int)base, tiles + (tile * 3 + q) * kTmaSubTileBytes);
+      bulk_commit();
+      if (NT == 1) bulk_wait_read<0>();                   // the tile may be overwritten (or the CTA may end) once it has been read
+      else if (!last) bulk_wait_read<1>();
+    }
+    if (!last) __syncthreads();
+  }
+};
 
 // ---------------------------------------------------------------------------------------------
 // K1, uniform S.  Output staging (MODE):
-//   kStageSpline  the 24 coefficients of ONE spline per thread go to shared memory [thread][25] (odd pitch in doubles:
-//                 a warp's 64-bit stores need the minimal 2 wavefronts) and leave the CTA after every spline, consecutive
-//                 threads writing consecutive doubles of the 192-byte (6-sector) chunk of each mission.  12.8 KB per CTA,
-//                 so residency is limited by registers only.
-//   kStagePair    the same with two splines per flush ([thread][49]): 384-byte chunks, i.e. whole 128-byte lines.
-//   kStageMission the whole mission ([thread][24 S + 1]) is staged and leaves as one contiguous tile (49.7 KB at S = 4).
+//   kStageCopy1, kStageCopy2  the 24 coefficients of MODE (one or two) splines per thread go to shared memory [thread][24 MODE + 1]
+//                 (odd pitch in doubles: a warp's 64-bit stores need the minimal 2 wavefronts) and leave the CTA by a copy loop after
+//                 every MODE splines, consecutive threads writing consecutive doubles of each mission's 192-byte (6-sector) or
+//                 384-byte (three whole 128-byte lines) chunk.  12.8 / 25 KB per CTA, so residency is limited by registers only.
+//   kStageTma     two splines per flush like kStageCopy2, but the tile leaves by tensor stores (SwizzledTiles<1>).
 //   kDirect       per-thread stores straight from registers (S > 8: work arrays in local memory anyway).
 // Threads past the end of the batch run the solve on the last mission (they must reach the barriers) and store nothing.
-//   kStageTma     two splines per flush like kStagePair, but the 64 x 48-double tile leaves the CTA as THREE 2-D tensor stores
-//                 (cp.async.bulk.tensor.2d, boxes of 64 missions x 16 doubles over the [B][24 S] coefficient matrix) issued by one
-//                 thread instead of a 48-iteration copy loop run by every thread; the tile is staged in the 128-byte swizzle
-//                 the tensor map declares (16-byte chunk c of row r at chunk c ^ (r & 7)), rows past the end of the batch and the
-//                 unused half of an odd last flush are clipped by the map.
-enum { kDirect = 0, kStageMission = 1, kStageSpline = 2, kStagePair = 3, kStageTma = 4 };
-constexpr int kTmaSubTileBytes = kSolveThreads * 128;     // 64 rows x 16 doubles
+enum { kDirect = 0, kStageCopy1 = 1, kStageCopy2 = 2, kStageTma = 3 };
 
 template <int MAXS, int MODE, int MINB>
 __global__ void __launch_bounds__(kSolveThreads, MINB) minsnap_solve_kernel(
@@ -50,74 +79,27 @@ __global__ void __launch_bounds__(kSolveThreads, MINB) minsnap_solve_kernel(
   auto loadw = [w](int i, int ax) { return __ldg(w + 3 * i + ax); };
   auto storet = [tout, live](int seg, double t) { if (live) tout[seg] = t; };
   int st;
-  if constexpr (MODE == kStageSpline) {
-    double* mine = s_out + (size_t)threadIdx.x * 25;
+  if constexpr (MODE == kStageCopy1 || MODE == kStageCopy2) {
+    constexpr int P = MODE, pitch = 24 * P + 1;          // splines per flush
+    double* mine = s_out + (size_t)threadIdx.x * pitch;
     double* gout = coeffs_out + (size_t)base * per;
     st = minsnap_solve_one<MAXS>(
-        S, velocity[bb], factor, loadw, [mine](int, int j, int ax, double val) { mine[j * 3 + ax] = val; }, storet,
+        S, velocity[bb], factor, loadw, [mine](int seg, int j, int ax, double val) { mine[(seg % P) * 24 + j * 3 + ax] = val; }, storet,
         [&](int seg) {
-          __syncthreads();
-          for (int e = threadIdx.x; e < n_here * 24; e += kSolveThreads) {
-            const int m = e / 24, off = e - m * 24;
-            gout[(size_t)m * per + seg * 24 + off] = s_out[m * 25 + off];
-          }
-          __syncthreads();
-        });
-  } else if constexpr (MODE == kStagePair) {
-    // two splines at a time: every mission leaves as 384-byte chunks = three whole 128-byte lines (mission stride 192 S bytes)
-    double* mine = s_out + (size_t)threadIdx.x * 49;
-    double* gout = coeffs_out + (size_t)base * per;
-    st = minsnap_solve_one<MAXS>(
-        S, velocity[bb], factor, loadw, [mine](int seg, int j, int ax, double val) { mine[(seg & 1) * 24 + j * 3 + ax] = val; }, storet,
-        [&](int seg) {
-          const bool last = seg == S - 1;
-          if (!(seg & 1) && !last) return;                 // uniform: S is the same for the whole launch
-          const int cnt = (seg & 1) ? 48 : 24, first = (seg & 1) ? seg - 1 : seg;
+          if (seg % P != P - 1 && seg != S - 1) return;    // uniform: S is the same for the whole launch
+          const int first = seg - seg % P, cnt = (seg % P + 1) * 24;
           __syncthreads();
           for (int e = threadIdx.x; e < n_here * cnt; e += kSolveThreads) {
             const int m = e / cnt, off = e - m * cnt;
-            gout[(size_t)m * per + first * 24 + off] = s_out[m * 49 + off];
+            gout[(size_t)m * per + first * 24 + off] = s_out[m * pitch + off];
           }
           __syncthreads();
         });
   } else if constexpr (MODE == kStageTma) {
-    char* tiles = reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(s_out) + 1023) & ~(uintptr_t)1023);      // 128-byte swizzle: 1024-byte aligned
-    char* row = tiles + threadIdx.x * 128;
-    const unsigned sw = (threadIdx.x & 7u) << 4;
+    const SwizzledTiles<1> tiles(reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(s_out) + 1023) & ~(uintptr_t)1023));   // 1024-byte aligned
     st = minsnap_solve_one<MAXS>(
-        S, velocity[bb], factor, loadw,
-        [row, sw](int seg, int j, int ax, double val) {
-          const int off = (seg & 1) * 24 + j * 3 + ax, q = off >> 4, d = off & 15;           // sub-tile, double within the 128-byte row
-          *reinterpret_cast<double*>(row + q * kTmaSubTileBytes + ((((unsigned)d >> 1) << 4) ^ sw) + (d & 1) * 8) = val;
-        },
-        storet,
-        [&](int seg) {
-          const bool last = seg == S - 1;
-          if (!(seg & 1) && !last) return;                 // uniform: S is the same for the whole launch
-          const int first = (seg & 1) ? seg - 1 : seg, n_sub = (seg & 1) ? 3 : 2;            // a lone last spline fills 24 of the 48 columns
-          fence_proxy_async_smem();
-          __syncthreads();
-          if (threadIdx.x == 0) {
-            for (int q = 0; q < n_sub; ++q) tensor_store_2d(&tmap, first * 24 + q * 16, (int)base, tiles + q * kTmaSubTileBytes);
-            bulk_commit();
-            bulk_wait_read<0>();                           // the tile may be overwritten (or the CTA may end) once it has been read
-          }
-          if (!last) __syncthreads();
-        });
-  } else if constexpr (MODE == kStageMission) {
-    const int pitch = per + 1;
-    double* mine = s_out + (size_t)threadIdx.x * pitch;
-    st = minsnap_solve_one<MAXS>(S, velocity[bb], factor, loadw, [mine](int seg, int j, int ax, double val) { mine[seg * 24 + j * 3 + ax] = val; }, storet);
-    __syncthreads();
-    double* gout = coeffs_out + (size_t)base * per;
-    const int total = n_here * per;
-    int mi = 0, off = threadIdx.x;       // e = mi * per + off, advanced without a division
-    while (off >= per) { off -= per; ++mi; }
-    for (int e = threadIdx.x; e < total; e += kSolveThreads) {
-      gout[e] = s_out[(size_t)mi * pitch + off];
-      off += kSolveThreads;
-      while (off >= per) { off -= per; ++mi; }
-    }
+        S, velocity[bb], factor, loadw, [tiles](int seg, int j, int ax, double val) { tiles.store(seg, j, ax, val); }, storet,
+        [&](int seg) { tiles.flush(&tmap, seg, S, base); });
   } else {
     double* mine = coeffs_out + (size_t)bb * per;
     st = minsnap_solve_one<MAXS>(S, velocity[bb], factor, loadw, [mine, live](int seg, int j, int ax, double val) { if (live) mine[seg * 24 + j * 3 + ax] = val; },
@@ -131,17 +113,9 @@ __global__ void __launch_bounds__(kSolveThreads, MINB) minsnap_solve_kernel(
 // (cp.async.bulk, completion on an mbarrier) while the current tile is solved, and the coefficients leave by tensor stores as in
 // kStageTma.  The one-shot kernels above start every CTA with a dependent global load of its waypoints (ncu: 4.2 long-scoreboard
 // stall cycles per issued instruction at 11 warps per SM); here a CTA waits for memory once, at its first tile.
-#ifndef UAVB_K1_STREAM_CTAS
-#define UAVB_K1_STREAM_CTAS 4
-#endif
-#ifndef UAVB_K1_STREAM_THREADS
-#define UAVB_K1_STREAM_THREADS 64
-#endif
-constexpr int kStreamCtasPerSm = UAVB_K1_STREAM_CTAS;
-constexpr int kStreamThreads = UAVB_K1_STREAM_THREADS;       // missions per tile
-constexpr int kStreamSubTileBytes = kStreamThreads * 128;
+constexpr int kStreamCtasPerSm = 4;
 template <int MAXS, int MINB>
-__global__ void __launch_bounds__(kStreamThreads, MINB) minsnap_solve_stream_kernel(
+__global__ void __launch_bounds__(kSolveThreads, MINB) minsnap_solve_stream_kernel(
     const double* __restrict__ waypoints, const double* __restrict__ velocity, int B, int S, double factor, double* __restrict__ times_out,
     int* __restrict__ status_out, const __grid_constant__ CUtensorMap tmap) {
   // Dynamic shared memory only (so that it starts 1024-byte aligned, as the 128-byte swizzle of the tensor stores needs): TWO staging
@@ -149,26 +123,24 @@ __global__ void __launch_bounds__(kStreamThreads, MINB) minsnap_solve_stream_ker
   // drain a tile before the next pair of splines is staged (the kernel is bound by HBM writes: that read-out waits for the write
   // queue) --, then the waypoints of the next tile, then the mbarrier: 56 840 bytes at S = 4, four CTAs per SM.
   extern __shared__ __align__(1024) double s_out[];
-  char* tiles = reinterpret_cast<char*>(s_out);
-  double* s_wp = reinterpret_cast<double*>(tiles + 6 * kStreamSubTileBytes);       // [64][3 (S+1)]
+  const SwizzledTiles<2> tiles(reinterpret_cast<char*>(s_out));
+  double* s_wp = reinterpret_cast<double*>(tiles.tiles + 6 * kTmaSubTileBytes);       // [64][3 (S+1)]
   const int wpd = 3 * (S + 1);
-  uint64_t* s_bar = reinterpret_cast<uint64_t*>(s_wp + kStreamThreads * 3 * (MAXS + 1));   // (a fixed place: behind the largest waypoint tile)
-  if ((smem_u32(tiles) & 1023u) != 0u) __trap();           // the staging tiles must sit on the swizzle period
-  char* row = tiles + threadIdx.x * 128;
-  const unsigned sw = (threadIdx.x & 7u) << 4;
-  const int n_tiles = (B + kStreamThreads - 1) / kStreamThreads;
+  uint64_t* s_bar = reinterpret_cast<uint64_t*>(s_wp + kSolveThreads * 3 * (MAXS + 1));   // (a fixed place: behind the largest waypoint tile)
+  if ((smem_u32(tiles.tiles) & 1023u) != 0u) __trap();     // the staging tiles must sit on the swizzle period
+  const int n_tiles = (B + kSolveThreads - 1) / kSolveThreads;
   // the waypoints of tile t: one bulk copy when the tile is whole, a cooperative copy for the ragged last tile (a bulk copy
   // needs a multiple of 16 bytes, 64 missions always are); the velocity of a thread's next mission travels in a register
   auto prefetch = [&](int tile) {                         // thread 0
-    if ((long long)(tile + 1) * kStreamThreads > B) return;
-    const uint32_t wp_bytes = (uint32_t)(kStreamThreads * wpd * 8);
+    if ((long long)(tile + 1) * kSolveThreads > B) return;
+    const uint32_t wp_bytes = (uint32_t)(kSolveThreads * wpd * 8);
     mbar_expect_tx(s_bar, wp_bytes);
-    bulk_load_1d(s_wp, waypoints + (size_t)tile * kStreamThreads * wpd, wp_bytes, s_bar);
+    bulk_load_1d(s_wp, waypoints + (size_t)tile * kSolveThreads * wpd, wp_bytes, s_bar);
   };
   auto velocity_of = [&](int tile) {                      // this thread's mission of `tile` (the tile's first one past the end of the batch)
     if (tile >= n_tiles) return 0.0;
-    const long long m = (long long)tile * kStreamThreads + threadIdx.x;
-    return __ldg(velocity + (m < B ? m : (long long)tile * kStreamThreads));
+    const long long m = (long long)tile * kSolveThreads + threadIdx.x;
+    return __ldg(velocity + (m < B ? m : (long long)tile * kSolveThreads));
   };
   if (threadIdx.x == 0) {
     mbar_init(s_bar, 1);
@@ -178,14 +150,14 @@ __global__ void __launch_bounds__(kStreamThreads, MINB) minsnap_solve_stream_ker
   __syncthreads();
   unsigned phase = 0;
   for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-    const long long base = (long long)tile * kStreamThreads;
-    const int n_here = (int)((B - base) < kStreamThreads ? (B - base) : kStreamThreads);
+    const long long base = (long long)tile * kSolveThreads;
+    const int n_here = (int)((B - base) < kSolveThreads ? (B - base) : kSolveThreads);
     const bool live = (int)threadIdx.x < n_here;
-    if (n_here == kStreamThreads) {
+    if (n_here == kSolveThreads) {
       mbar_wait(s_bar, phase);
       phase ^= 1u;
     } else {                                              // ragged last tile (the last iteration of one CTA)
-      for (int e = threadIdx.x; e < n_here * wpd; e += kStreamThreads) s_wp[e] = __ldg(waypoints + (size_t)base * wpd + e);
+      for (int e = threadIdx.x; e < n_here * wpd; e += kSolveThreads) s_wp[e] = __ldg(waypoints + (size_t)base * wpd + e);
       __syncthreads();
     }
     // this thread's mission into registers (threads past the end of the batch solve the tile's first mission and store nothing)
@@ -202,24 +174,9 @@ __global__ void __launch_bounds__(kStreamThreads, MINB) minsnap_solve_stream_ker
     double* tout = times_out + (size_t)(base + src) * S;
     const int st = minsnap_solve_one<MAXS>(
         S, vel, factor, [&wreg](int i, int ax) { return wreg[3 * i + ax]; },
-        [row, sw](int seg, int j, int ax, double val) {
-          const int off = (seg & 1) * 24 + j * 3 + ax, q = off >> 4, d = off & 15, half = (seg >> 1) & 1;
-          *reinterpret_cast<double*>(row + (half * 3 + q) * kStreamSubTileBytes + ((((unsigned)d >> 1) << 4) ^ sw) + (d & 1) * 8) = val;
-        },
+        [tiles](int seg, int j, int ax, double val) { tiles.store(seg, j, ax, val); },
         [tout, live](int seg, double t) { if (live) tout[seg] = t; },
-        [&](int seg) {
-          const bool last = seg == S - 1;
-          if (!(seg & 1) && !last) return;
-          const int first = (seg & 1) ? seg - 1 : seg, n_sub = (seg & 1) ? 3 : 2, half = (seg >> 1) & 1;
-          fence_proxy_async_smem();
-          __syncthreads();
-          if (threadIdx.x == 0) {
-            for (int q = 0; q < n_sub; ++q) tensor_store_2d(&tmap, first * 24 + q * 16, (int)base, tiles + (half * 3 + q) * kStreamSubTileBytes);
-            bulk_commit();
-            if (!last) bulk_wait_read<1>();               // the OTHER staging tile's last store (a whole tile ago) has read it: it is staged next
-          }
-          if (!last) __syncthreads();
-        });
+        [&](int seg) { tiles.flush(&tmap, seg, S, base); });
     if (live && status_out) status_out[base + threadIdx.x] = st;
   }
   if (threadIdx.x == 0) bulk_wait_read<0>();              // shared memory must outlive the last store's read
@@ -656,19 +613,15 @@ __global__ void __launch_bounds__(128) constraint_rows_kernel(const double* __re
 template <int MAXS, int MODE, int MINB>
 static int launch_solve(const double* w, const double* vel, int B, int S, double factor, double* c, double* t, int* st, cudaStream_t stream,
                         const CUtensorMap* tmap = nullptr) {
-  const size_t smem = MODE == kStageMission ? sizeof(double) * (size_t)kSolveThreads * (24 * S + 1)
-                                            : (MODE == kStageSpline ? sizeof(double) * (size_t)kSolveThreads * 25
-                                               : (MODE == kStagePair ? sizeof(double) * (size_t)kSolveThreads * 49
-                                                  : (MODE == kStageTma ? (size_t)3 * kTmaSubTileBytes + 1024 : 0)));
-  if (smem > 48 * 1024)
-    UAVB_CUDA_OK(cudaFuncSetAttribute(minsnap_solve_kernel<MAXS, MODE, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const size_t smem = MODE == kStageTma ? (size_t)3 * kTmaSubTileBytes + 1024
+                                        : (MODE == kDirect ? 0 : sizeof(double) * (size_t)kSolveThreads * (24 * MODE + 1));   // kStageCopy1/2
   CUtensorMap none = {};
   minsnap_solve_kernel<MAXS, MODE, MINB><<<div_up(B, kSolveThreads), kSolveThreads, smem, stream>>>(w, vel, B, S, factor, c, t, st, tmap ? *tmap : none);
   UAVB_CUDA_OK(cudaGetLastError());
   return UAVB_OK;
 }
 
-// The [B][24 S] coefficient matrix as a tensor map with boxes of 64 missions x 16 doubles in the 128-byte swizzle (kStageTma).
+// The [B][24 S] coefficient matrix as a tensor map with boxes of 64 missions x 16 doubles in the 128-byte swizzle (SwizzledTiles).
 static bool coeff_tensor_map(CUtensorMap* tm, double* coeffs, int B, int S) {
   return make_tensor_map_2d(tm, coeffs, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 24ull * S, (unsigned long long)B, 192ull * S, 16, kSolveThreads,
                             CU_TENSOR_MAP_SWIZZLE_128B);
@@ -687,55 +640,22 @@ extern "C" int uavb_minsnap_solve_f64(const double* waypoints, const double* vel
   if (rc) return rc;
   if (B == 0) return UAVB_OK;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-#ifdef UAVB_DEV
-  if (const char* dev_mode = getenv("UAVB_K1_VARIANT")) {             // development override: staging / residency experiments at S <= 4
-    const int v = atoi(dev_mode);
-    if (S <= 4 && S > 2) {
-      switch (v) {
-        case 1: return launch_solve<4, kStageMission, 1>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st);
-        case 2: return launch_solve<4, kStageSpline, 1>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st);
-        case 3: return launch_solve<4, kStageSpline, 6>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st);
-        case 4: return launch_solve<4, kStageSpline, 8>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st);
-        case 5: return launch_solve<4, kDirect, 1>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st);
-        case 6: return launch_solve<4, kDirect, 8>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st);
-        case 7: return launch_solve<4, kStageSpline, 10>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st);
-        case 8: return launch_solve<4, kStagePair, 6>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st);
-        case 9: {
-          CUtensorMap tmv;
-          if (coeff_tensor_map(&tmv, coeffs_out, B, S)) return launch_solve<4, kStageTma, 8>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st, &tmv);
-          break;
-        }
-        default: break;
-      }
-    }
-  }
-#endif
-  if (S == 1) return launch_solve<1, kStageSpline, 1>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st);
-  if (S == 2) return launch_solve<2, kStageSpline, 1>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st);
+  if (S == 1) return launch_solve<1, kStageCopy1, 1>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st);
+  if (S == 2) return launch_solve<2, kStageCopy1, 1>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st);
   // S <= 4 (BASELINE configs[1]): 6 CTAs per SM (168 registers) measured fastest -- 0.216 ms per 10^6 solves against 0.250 ms
-  // unconstrained (198 registers, 5 CTAs) and 0.238 ms at 8 CTAs (128 registers, spills); tools/k1_sweep.sh
+  // unconstrained (198 registers, 5 CTAs) and 0.238 ms at 8 CTAs (128 registers, spills); DESIGN.md, K1
   // ... and staging two splines at a time (384-byte chunks = whole 128-byte lines, 25 KB per CTA) 0.198 ms against 0.2026 ms
   // ... and, where the driver gives a tensor map (16-byte aligned output), the tile leaves through the TMA unit instead of a copy loop
   CUtensorMap tm;
   const bool tma = S > 2 && S <= 8 && coeff_tensor_map(&tm, coeffs_out, B, S);
-  bool streaming = tma && S == 4 &&     // measured: S = 3 is 5 % faster one-shot (6 CTAs per SM), S = 4 14 % faster streaming
-                   (reinterpret_cast<uintptr_t>(waypoints) & 15u) == 0 && (reinterpret_cast<uintptr_t>(velocity) & 15u) == 0;
-#ifdef UAVB_DEV
-  if (getenv("UAVB_K1_ONESHOT")) streaming = false;           // development builds only: the one-shot tensor-store kernel for comparison
-#endif
+  const bool streaming = tma && S == 4 &&     // measured: S = 3 is 5 % faster one-shot (6 CTAs per SM), S = 4 14 % faster streaming
+                         (reinterpret_cast<uintptr_t>(waypoints) & 15u) == 0 && (reinterpret_cast<uintptr_t>(velocity) & 15u) == 0;
   if (streaming) {
     int sms = 0;
     rc = sm_count_cached(&sms);
     if (rc) return rc;
-    const size_t smem = (size_t)6 * kStreamSubTileBytes + sizeof(double) * kStreamThreads * 3 * (4 + 1) + sizeof(uint64_t);   // MAXS = 4
-    const int n_tiles = div_up(B, kStreamThreads);
-    CUtensorMap tms;
-    if (kStreamThreads != kSolveThreads) {                 // the streaming kernel's tile has its own box height
-      if (!make_tensor_map_2d(&tms, coeffs_out, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 24ull * S, (unsigned long long)B, 192ull * S, 16, kStreamThreads,
-                              CU_TENSOR_MAP_SWIZZLE_128B))
-        return set_error(UAVB_ECUDA, "minsnap_solve: tensor map");
-      tm = tms;
-    }
+    const size_t smem = (size_t)6 * kTmaSubTileBytes + sizeof(double) * kSolveThreads * 3 * (4 + 1) + sizeof(uint64_t);   // MAXS = 4
+    const int n_tiles = div_up(B, kSolveThreads);
     const int grid = n_tiles < kStreamCtasPerSm * sms ? n_tiles : kStreamCtasPerSm * sms;
     static std::once_flag attr_once[kMaxDevices];          // > 48 KB of dynamic shared memory needs the opt-in, once per device
     int dev = 0;
@@ -747,17 +667,17 @@ extern "C" int uavb_minsnap_solve_f64(const double* waypoints, const double* vel
         attr_err = cudaFuncSetAttribute(minsnap_solve_stream_kernel<4, kStreamCtasPerSm>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     });
     UAVB_CUDA_OK(attr_err);
-    minsnap_solve_stream_kernel<4, kStreamCtasPerSm><<<grid, kStreamThreads, smem, st>>>(waypoints, velocity, B, S, factor, times_out, status_out, tm);
+    minsnap_solve_stream_kernel<4, kStreamCtasPerSm><<<grid, kSolveThreads, smem, st>>>(waypoints, velocity, B, S, factor, times_out, status_out, tm);
     UAVB_CUDA_OK(cudaGetLastError());
     return UAVB_OK;
   }
   if (S <= 4) {
     if (tma) return launch_solve<4, kStageTma, 6>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st, &tm);
-    return launch_solve<4, kStagePair, 6>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st);
+    return launch_solve<4, kStageCopy2, 6>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st);
   }
   if (S <= 8) {
     if (tma) return launch_solve<8, kStageTma, 1>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st, &tm);
-    return launch_solve<8, kStageSpline, 1>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st);
+    return launch_solve<8, kStageCopy1, 1>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st);
   }
   return launch_solve<UAVB_MAX_SPLINES, kDirect, 1>(waypoints, velocity, B, S, factor, coeffs_out, times_out, status_out, st);
 }
