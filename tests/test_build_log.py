@@ -1,7 +1,7 @@
 """Guards on what ptxas made of the hot kernels (uav-autonomous-control_b200/lib/build.log, written by build.py): the persistent
 rollout kernels must not keep state in local memory.  (Round 2: one extra inlined call site of the flying code made ptxas copy the
 kernel parameter block to the stack in six of eight instantiations -- 1280-byte frames, BASELINE configs[3] 108 -> 191 ms -- without
-any test noticing.)"""
+any test noticing.)  Also: what the built library itself contains."""
 from __future__ import annotations
 
 import os
@@ -11,6 +11,7 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LOG = os.path.join(ROOT, "uav-autonomous-control_b200", "lib", "build.log")
+LIB = os.path.join(ROOT, "uav-autonomous-control_b200", "lib", "libuavb.so")
 
 
 def _kernels():
@@ -35,3 +36,12 @@ def test_rollout_kernels_keep_their_state_in_registers():
 def test_streaming_solver_fits_four_ctas_per_sm():
     ks = [k for k in _kernels() if "minsnap_solve_stream_kernelILi4" in k[0]]
     assert ks and ks[0][3] <= 255 and ks[0][2] <= 64             # 4 CTAs x 64 threads x 255 registers; a handful of spilled bytes at most
+
+
+@pytest.mark.skipif(not os.path.exists(LIB), reason="library not built in this tree")
+def test_library_reads_no_slicing_overrides_from_the_environment():
+    """How a rollout launch is sliced is fixed in the code: no variable in the user's environment changes it."""
+    with open(LIB, "rb") as f:
+        data = f.read()
+    for name in (b"UAVB_ROLLOUT_CHUNKS", b"UAVB_SLICE_MIN", b"UAVB_SLICE_PART"):
+        assert name not in data, name.decode()

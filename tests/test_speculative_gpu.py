@@ -22,11 +22,11 @@ def spec(cuda):
     """force(flag): fly every stretch of the speculative kernels with the exact body (1) or speculate (0)."""
     from uav_ac_b200 import _native as nat
     fn = nat.lib().uavb_dev_speculation
-    fn.argtypes = [ctypes.c_int, ctypes.c_void_p, ctypes.c_int]
+    fn.argtypes = [ctypes.c_int]
     fn.restype = ctypes.c_int
 
     def force(flag):
-        assert fn(int(flag), None, 0) == 0
+        assert fn(int(flag)) == 0
     yield force
     force(0)
 

@@ -1,7 +1,5 @@
 #!/bin/bash
-# usage: clk.sh <tag> <B> <reps>
-lib=uav-autonomous-control_b200/lib/libuavb.so
-[ "$1" != default ] && cp build/variants/libuavb_$1.so $lib
+# usage: clk_probe.sh <tag> <B> <reps>   (tag names the output file clk_<tag>.csv)
 nvidia-smi --query-gpu=clocks.sm,power.draw,clocks_event_reasons.active,clocks_event_reasons.sw_power_cap,clocks_event_reasons.hw_slowdown,clocks_event_reasons.sw_thermal_slowdown,temperature.gpu --format=csv,noheader -lms 100 > gpurun_out/clk_$1.csv &
 SMI=$!
 python tools/k2_probe.py $2 $3

@@ -11,7 +11,7 @@ per arm, with the card's name and power limit read in the same run.
 
 A 256 MB buffer is written between timed passes (L2 flush).  steps/s = rollouts x ticks / kernel time; table_bytes_per_s = the
 set-point records the kernel reads (56 B per rollout and outer period) / kernel time -- for arm a every rollout reads the same
-60 kB, so that figure is L1/L2 traffic, not HBM.  --lib flies a variant build of the library (build.py --variant).
+60 kB, so that figure is L1/L2 traffic, not HBM.  --lib flies another build of the library, e.g. a parent commit's libuavb.so.
 """
 from __future__ import annotations
 

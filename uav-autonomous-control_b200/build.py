@@ -42,29 +42,6 @@ def _fingerprint() -> str:
     return h.hexdigest()
 
 
-def build_variant(tag: str, defines: list[str]) -> str:
-    """Development aid: the same library with extra -D flags, as build/variants/libuavb_<tag>.so (not loaded by the package)."""
-    out = os.path.join(ROOT, "build", "variants", f"libuavb_{tag}.so")
-    objdir = os.path.join(ROOT, "build", "variants", tag)
-    os.makedirs(objdir, exist_ok=True)
-    procs, objs = [], []
-    for src in SOURCES:
-        obj = os.path.join(objdir, src.replace(".cu", ".o"))
-        procs.append((src, subprocess.Popen([_nvcc(), *NVCC_FLAGS, *defines, "-Xptxas", "-v", "-c", os.path.join(CSRC, src), "-o", obj],
-                                            stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
-        objs.append(obj)
-    log = []
-    for src, p in procs:
-        o, _ = p.communicate()
-        log.append(o)
-        if p.returncode != 0:
-            raise RuntimeError(f"nvcc failed on {src}:\n{o}")
-    subprocess.run([_nvcc(), "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-o", out, *objs], check=True)
-    with open(os.path.join(objdir, "build.log"), "w") as f:
-        f.write("\n".join(log))
-    return out
-
-
 def build(force: bool = False, verbose: bool = False) -> str:
     os.makedirs(LIBDIR, exist_ok=True)
     stamp = os.path.join(LIBDIR, "libuavb.stamp")
@@ -101,8 +78,4 @@ def build(force: bool = False, verbose: bool = False) -> str:
 
 
 if __name__ == "__main__":
-    if "--variant" in sys.argv:                       # build.py --variant <tag> -DNAME=VALUE ...
-        i = sys.argv.index("--variant")
-        print(build_variant(sys.argv[i + 1], sys.argv[i + 2:]))
-    else:
-        print(build(force="--force" in sys.argv, verbose="--verbose" in sys.argv))
+    print(build(force="--force" in sys.argv, verbose="--verbose" in sys.argv))

@@ -221,16 +221,10 @@ template <bool NORM, bool LAG, class VP> UAVB_DEV void inner_tick_pair(Drone2& d
 
 // The speculative tick (rollout_run_pair): inner_tick_pair<false, LAG> without its two rare paths and without a branch.  It always
 // keeps the unclipped mixer outputs and the tan-form quaternion map; a lane where the exact tick would take the rotor-limit path
-// (failed sufficient test) or the large-rotation path (|w|^2 >= small_rot_wn2) sets its bit in `rare`, and its state is then wrong.
-// Where no bit is set the tick ran exactly the rounded operations of inner_tick_pair<false, LAG>, so the two must change together.
+// (failed sufficient test) or the large-rotation path (|w|^2 >= small_rot_wn2) sets `rare`, and its state is then wrong.
+// Where `rare` stays 0 the tick ran exactly the rounded operations of inner_tick_pair<false, LAG>, so the two must change together.
 // (A copy rather than a template switch of inner_tick_pair: as a switch, the same operations reach ptxas in another order and the
 // speculative kernels compile to different machine code.)
-// Bits of `rare`: one for both paths unless a counting build (UAVB_SPEC_COUNT, development only) tells them apart.
-#ifndef UAVB_SPEC_COUNT
-#define UAVB_SPEC_COUNT 0
-#endif
-constexpr int kRareLimitBit = 0;
-constexpr int kRareRotBit = UAVB_SPEC_COUNT ? 1 : 0;
 template <bool LAG, class VP> UAVB_DEV void inner_tick_pair_spec(Drone2& d, const VehU<float>& u, const VP& v, unsigned& rare) {
   const V2 yz = mul2(d.wy, d.wz), zx = mul2(d.wz, d.wx), xy = mul2(d.wx, d.wy);
   // mixer butterfly of mix_and_limit_pair, its sufficient test recorded instead of branched on
@@ -238,7 +232,7 @@ template <bool LAG, class VP> UAVB_DEV void inner_tick_pair_spec(Drone2& d, cons
   const V2 rb = fma2(neg2(v.Jr), d.wz, fma2(v.Gz, xy, d.cr));
   const V2 m1 = add2(pb, qb), m2 = sub2(pb, qb), t1 = add2(d.coll, rb), t2 = sub2(d.coll, rb);
   const V2 need = add2(add2(abs2(pb), abs2(qb)), abs2(rb));
-  rare |= (unsigned)(!(need.x <= d.margin.x) | !(need.y <= d.margin.y)) << kRareLimitBit;
+  rare |= (unsigned)(!(need.x <= d.margin.x) | !(need.y <= d.margin.y));
   lag_toward_pair(d, u, sqrt2(add2(t1, m1)), sqrt2(sub2(t2, m2)), sqrt2(sub2(t1, m1)), sqrt2(add2(t2, m2)));
   V2 ha, hb, hc;
   half_axis_pair(d, ha, hb, hc);
@@ -265,7 +259,7 @@ template <bool LAG, class VP> UAVB_DEV void inner_tick_pair_spec(Drone2& d, cons
   const V2 sf = fma2(wn2, u.half_dt_cu3, u.half_dt);
   const V2 bx = mul2(sf, d.wx), by = mul2(sf, d.wy), bz = mul2(sf, d.wz);
   const V2 q0 = d.q0, q1 = d.q1, q2 = d.q2, q3 = d.q3;
-  rare |= (unsigned)(!(wn2.x < u.small_rot_wn2) | !(wn2.y < u.small_rot_wn2)) << kRareRotBit;
+  rare |= (unsigned)(!(wn2.x < u.small_rot_wn2) | !(wn2.y < u.small_rot_wn2));
   d.q0 = sub2(q0, fma2(q3, bz, fma2(q2, by, mul2(q1, bx))));
   d.q1 = add2(q1, fma2(neg2(q3), by, fma2(q2, bz, mul2(q0, bx))));
   d.q2 = add2(q2, fma2(q3, bx, fma2(neg2(q1), bz, mul2(q0, by))));

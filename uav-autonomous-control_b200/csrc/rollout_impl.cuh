@@ -32,11 +32,9 @@ namespace uavb {
 //     only adds waiting at that barrier.
 //   * rollouts with a state log: 64 threads (128 drones), 4 CTAs per SM -- a CTA writes 512 contiguous bytes per field and sample.
 //   * fp64 validation build: one drone per thread, 64 threads, one-shot launch, 128 registers.
-#ifndef UAVB_PAIR_REGS
-#define UAVB_PAIR_REGS 255
-#endif
-constexpr int kRolloutPairRegs = UAVB_PAIR_REGS;      // fp32 production build
-constexpr int kPairWarpsPerSm = 65536 / (32 * ((UAVB_PAIR_REGS + 15) / 16 * 16));   // registers are allocated in units of 16 per thread
+// 9 or 10 warps per SM at 224 / 208 / 192 registers and 12 at 168 measured slower (DESIGN.md, K2 round 2).
+constexpr int kRolloutPairRegs = 255;
+constexpr int kPairWarpsPerSm = 65536 / (32 * ((kRolloutPairRegs + 15) / 16 * 16));   // registers are allocated in units of 16 per thread
 constexpr int kRolloutThreads = 32;
 constexpr int kRolloutCtasPerSm = kPairWarpsPerSm;
 constexpr int kRolloutThreadsLog = 64;
@@ -632,23 +630,6 @@ __global__ void __maxnreg__(kRolloutPairRegs) rollout_sliced_tables_tma_kernel(c
 
 // Development switch of the speculative bodies (rollout_pair.cuh, set by uavb_dev_speculation): fly every stretch exactly.
 extern int g_spec_exact;
-// Counting builds (UAVB_SPEC_COUNT): read (and zero) the stretch counters of one translation unit (8 words; zeros otherwise).
-cudaError_t spec_counts_sliced(unsigned long long* counts, bool reset);
-cudaError_t spec_counts_tables(unsigned long long* counts, bool reset);
-template <int TU> static cudaError_t spec_counts(unsigned long long* counts, bool reset) {
-#if UAVB_SPEC_COUNT
-  cudaError_t e = cudaMemcpyFromSymbol(counts, g_spec_count, sizeof(g_spec_count));
-  if (e == cudaSuccess && reset) {
-    const unsigned long long z[8] = {};
-    e = cudaMemcpyToSymbol(g_spec_count, z, sizeof(z));
-  }
-  return e;
-#else
-  (void)reset;
-  for (int k = 0; k < 8; ++k) counts[k] = 0;
-  return cudaSuccess;
-#endif
-}
 
 // Launch of a pair kernel: MODE (kTargetFly / kTargetShared / kTargetPerRollout, `ts` required for the last) and LOG (as pair_slice;
 // 2 requires `maps`) pick the kernel family and its CTA shape, mc and lag its instantiation.  Each (MODE, LOG) is instantiated by the

@@ -2,10 +2,6 @@
 // shared mission, and the C entry points.  The device code lives in rollout_impl.cuh; its kernels are instantiated, with their
 // launchers, in rollout_sliced.cu / rollout_log.cu / rollout_traj.cu / rollout_tables.cu / rollout_tables_log.cu (two drones per
 // thread), rollout_scalar.cu (one drone per thread) and rollout_f64.cu (fp64 validation build).
-#ifdef UAVB_DEV
-#include <stdlib.h>
-#endif
-
 #include "rollout_impl.cuh"
 
 namespace uavb {
@@ -160,12 +156,6 @@ template <class R> static int launch_rollout(const uavb_rollout_args* a, void* s
     // ~32 items per resident CTA keep the tail near 3 % of the launch; slices are whole outer periods of >= 100 ticks
     constexpr int kMinChunkTicks = 100;
     long long want = grid > slots ? (32LL * slots + grid - 1) / grid : 1;
-#ifdef UAVB_DEV
-    if (const char* force = getenv("UAVB_ROLLOUT_CHUNKS")) {       // development builds only (build.py --variant dev -DUAVB_DEV): force the slice count
-      const int f = atoi(force);
-      if (f > 0) want = f < 4096 ? f : 4096;
-    }
-#endif
     if (a->n_slices > 0) want = a->n_slices < 4096 ? a->n_slices : 4096;         // uavb.h: results are independent of the slice count
     const int period = a->inner_per_outer;
     int chunk = (int)((a->n_ticks + want - 1) / want);
@@ -201,21 +191,18 @@ template <class R> static int launch_rollout(const uavb_rollout_args* a, void* s
     // (whole outer periods), down to a length that is <= 0.5 % of a resident CTA's share of the launch and >= 200 ticks.  Measured on the
     // headline launch (1e5 x 10 760 ticks, 1 563 groups on 1 184 resident CTAs): 15 such slices 4.605 ms against 4.653 ms for the 25 equal
     // slices of the rule above (tools/pipeline_probe.py).  Results do not depend on the slicing (tests/test_rollout_gpu.py).
+    // The two constants sit on a flat optimum: fractions 1/3 ... 1/8 with floors of 100 ... 400 ticks land within +-0.7 % (DESIGN.md).
+    constexpr int kSlicePart = 5, kSliceFloorTicks = 200;
     if (a->n_slices <= 0 && n_chunks > 1) {
       const double share = (double)grid / (double)slots * (double)a->n_ticks;       // ticks a resident CTA flies in this launch
       int min_len = share / 200.0 < (double)a->n_ticks ? (int)(share / 200.0) : a->n_ticks;     // (never longer than the launch: no overflow below)
-      int floor_len = 200, part = 5;
-#ifdef UAVB_DEV
-      if (const char* e = getenv("UAVB_SLICE_MIN")) floor_len = atoi(e) > 0 ? atoi(e) : floor_len;      // development builds only
-      if (const char* e = getenv("UAVB_SLICE_PART")) part = atoi(e) > 1 ? atoi(e) : part;
-#endif
-      if (min_len < floor_len) min_len = floor_len;
+      if (min_len < kSliceFloorTicks) min_len = kSliceFloorTicks;
       min_len = (int)(((long long)min_len + period - 1) / period * period);
       int t = 0, n = 0;
       sch.tab[0] = 0;
       while (t < a->n_ticks) {
         const int left = a->n_ticks - t;
-        int len = left / part;
+        int len = left / kSlicePart;
         if (len < min_len) len = min_len;
         const long long whole = ((long long)len + period - 1) / period * period;      // whole outer periods
         len = whole < left ? (int)whole : left;
@@ -228,7 +215,7 @@ template <class R> static int launch_rollout(const uavb_rollout_args* a, void* s
     }
     // metrics-only shared-table / per-rollout-table bodies: the speculative stretches' checkpoints (rollout_pair.cuh), 160 B per thread
     // after the staged boxes -- 5 KB per one-warp CTA, 8 CTAs per SM stay resident
-    if (!log && a->traj_out == nullptr && !scalar32 && (from_table || tabs) && UAVB_SPECULATE) {
+    if (!log && a->traj_out == nullptr && !scalar32 && (from_table || tabs)) {
       smem = (smem + 15) / 16 * 16;
       smem += sizeof(float4) * kSpecSlotVec4 * threads;
     }
@@ -352,20 +339,9 @@ extern "C" int uavb_rollout_targets_f64(const double* seg_coeffs, const int* seg
 }
 
 // Development entry point, not part of uavb.h (tests/test_speculative_gpu.py, tools/spec_probe.py): force_exact = 1 flies every
-// stretch of the speculative kernels with the exact body in later launches, 0 restores speculation (< 0: unchanged);
-// counts (8 words, may be NULL) receives the stretch counters of a counting build (UAVB_SPEC_COUNT), summed over the kernels, and
-// reset = 1 zeroes them.
-extern "C" int uavb_dev_speculation(int force_exact, unsigned long long* counts, int reset) {
-  using namespace uavb;
-  if (force_exact >= 0) g_spec_exact = force_exact != 0;
-  if (!counts && !reset) return UAVB_OK;
-  int rc = require_device();
-  if (rc) return rc;
-  unsigned long long c0[8], c1[8];
-  UAVB_CUDA_OK(spec_counts_sliced(c0, reset != 0));
-  UAVB_CUDA_OK(spec_counts_tables(c1, reset != 0));
-  if (counts)
-    for (int k = 0; k < 8; ++k) counts[k] = c0[k] + c1[k];
+// stretch of the speculative kernels with the exact body in later launches, 0 restores speculation.
+extern "C" int uavb_dev_speculation(int force_exact) {
+  uavb::g_spec_exact = force_exact != 0;
   return UAVB_OK;
 }
 

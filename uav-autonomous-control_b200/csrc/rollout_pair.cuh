@@ -14,13 +14,11 @@
 
 #include <type_traits>
 
-#ifndef UAVB_TICK_UNROLL
-#define UAVB_TICK_UNROLL 2
-#endif
-
 namespace uavb {
 
-constexpr int kTickUnroll = UAVB_TICK_UNROLL;
+// Ticks per loop iteration of the unrolled bodies (rollout_run_pair): 2 beats 1 by 2 % on the headline launch and by 1-2 % with
+// per-rollout tables (DESIGN.md), and beats 5 / 10 in the speculative loop (profiles/r03_spec_probe.jsonl: 4.40 against 4.43 / 4.54 ms).
+constexpr int kTickUnroll = 2;
 
 // [sample][13][B] state log of a pair: drones 2j, 2j+1 are neighbours in every field row, so a field leaves as ONE 8-byte
 // streaming store per thread when the rows are 8-byte aligned (B even) -- a warp writes 256 contiguous bytes per field.
@@ -152,38 +150,17 @@ struct NoPairLog {
 //                      (N, 11) trajectory tables converted by uavb_table_targets_f64.
 enum : int { kTargetFly = 0, kTargetShared = 1, kTargetPerRollout = 2 };
 
-// Per-rollout tables: prefetch each lane's row of the NEXT outer period into L1 (as the shared-table body does for its one row),
-// and ticks per iteration of their metrics-only bodies (tools/table_probe.py measures both against the alternatives).
-#ifndef UAVB_TABLES_PREFETCH
-#define UAVB_TABLES_PREFETCH 1
-#endif
-#ifndef UAVB_TABLES_TICK_UNROLL
-#define UAVB_TABLES_TICK_UNROLL UAVB_TICK_UNROLL
-#endif
-constexpr int kTablesTickUnroll = UAVB_TABLES_TICK_UNROLL;
-
 // Speculative stretches (metrics-only bodies of the shared-table and per-rollout-table modes).  The exact tick carries two rare
 // paths -- the rotor-limit path and the large-rotation quaternion map -- and the branch around each keeps the next tick's head
 // from being scheduled against this tick's body.  A non-watching stretch therefore flies the branch-free inner_tick_pair_spec, with
 // the fields the tick writes checkpointed in shared memory first; when some lane of the warp would have taken a rare path, the warp
 // reloads the checkpoint and flies the same ticks with the exact body.  Without a rare path both bodies execute the same rounded
-// operations, so results are bit-identical either way.
-//   UAVB_SPECULATE    0 = always the exact body (the kernels of the previous release)
-//   UAVB_SPEC_HOLD    non-watching stretches flown with the exact body after a rollback (rare paths cluster in mission phases)
-//   UAVB_SPEC_UNROLL  ticks per iteration of the speculative loop
-#ifndef UAVB_SPECULATE
-#define UAVB_SPECULATE 1
-#endif
-#ifndef UAVB_SPEC_HOLD
-#define UAVB_SPEC_HOLD 4
-#endif
-#ifndef UAVB_SPEC_UNROLL
-#define UAVB_SPEC_UNROLL 2
-#endif
-constexpr int kSpecHold = UAVB_SPEC_HOLD;
-constexpr int kSpecUnroll = UAVB_SPEC_UNROLL;
+// operations, so results are bit-identical either way.  Measured in DESIGN.md (K2, speculative stretches).
+// Non-watching stretches flown with the exact body after a rollback (rare paths cluster in mission phases): 4 against 0 / 16 gives
+// 4.40 against 4.64 / 4.41 ms (profiles/r03_spec_probe.jsonl).
+constexpr int kSpecHold = 4;
 constexpr int kSpecSlotVec4 = 10;                            // 20 float2 fields of Drone2 = 10 x 16 bytes per thread
-template <int MODE, class LOG> constexpr bool kSpecBody = UAVB_SPECULATE && std::is_same<LOG, NoPairLog>::value && MODE != kTargetFly;
+template <int MODE, class LOG> constexpr bool kSpecBody = std::is_same<LOG, NoPairLog>::value && MODE != kTargetFly;
 
 // One thread's checkpoint in dynamic shared memory: 16-byte words k = 0..9 at s_spec[base + 32 k], base = the slot area (after the
 // staged boxes) + 320 words per warp + the lane -- a warp's store of one word is 512 contiguous bytes, conflict-free, and the
@@ -219,12 +196,6 @@ struct SpecSlot {
     t = w(9); d.zby = make_float2(t.x, t.y); d.zbz = make_float2(t.z, t.w);
   }
 };
-
-// Counting builds (UAVB_SPEC_COUNT, development only): per-warp counts of the stretches [watching, non-watching, speculated, rolled
-// back, some lane failed the sufficient rotor-limit test, some lane had a large rotation], one copy per translation unit.
-#if UAVB_SPEC_COUNT
-static __device__ unsigned long long g_spec_count[8];
-#endif
 
 // Set-points of the coming outer period and the position errors (set-point - position, fp64, rounded once): one table row
 // for both lanes of a shared mission, otherwise each lane's own cursor or table.
@@ -274,14 +245,13 @@ template <> struct PairTarget<kTargetPerRollout> {
     if (c[0].row + 1 < ma.n_trows) ++c[0].row;               // index clamp of main.py:61, with the lane's own row count
     table_target<float>(mb.trows, c[1].row, &tb);
     if (c[1].row + 1 < mb.n_trows) ++c[1].row;
-#if UAVB_TABLES_PREFETCH
+    // each lane's row of the NEXT outer period into L1, as for the shared table: 5 % once the tables leave L2 (DESIGN.md)
     const char* na = reinterpret_cast<const char*>(ma.trows + c[0].row);
     const char* nb = reinterpret_cast<const char*>(mb.trows + c[1].row);
     asm volatile("prefetch.global.L1 [%0];" ::"l"(na));
     asm volatile("prefetch.global.L1 [%0];" ::"l"(na + sizeof(TargetRow) - 4));
     asm volatile("prefetch.global.L1 [%0];" ::"l"(nb));
     asm volatile("prefetch.global.L1 [%0];" ::"l"(nb + sizeof(TargetRow) - 4));
-#endif
     zip_targets(d, ta, tb, t2, ex, ey, ez);
   }
 };
@@ -363,7 +333,7 @@ UAVB_DEV void rollout_run_pair(Drone2& d, Cursor<float> (&c)[2], Accum<float> (&
       // waits for instruction fetches and runs 10 % slower (measured).  Per-rollout tables unroll only without a state log: with
       // Monte-Carlo overrides and per-thread log stores the unrolled body no longer fits 255 registers (ptxas spills), and a
       // logging launch is bound by its HBM stores anyway.
-#pragma unroll((kWatch || MODE == kTargetFly) ? 1 : MODE == kTargetShared ? kTickUnroll : LOG::kNormEveryTick ? 1 : kTablesTickUnroll)
+#pragma unroll((kWatch || MODE == kTargetFly || (MODE == kTargetPerRollout && LOG::kNormEveryTick)) ? 1 : kTickUnroll)
       for (int j = 0; j < n; ++j) {
         inner_tick_pair<LOG::kNormEveryTick, LAG>(d, u, v2);
         if constexpr (kWatch) {
@@ -379,28 +349,15 @@ UAVB_DEV void rollout_run_pair(Drone2& d, Cursor<float> (&c)[2], Accum<float> (&
       if (!watch && hold == 0) {                             // (warp-uniform)
         slot.save(d);
         unsigned rare = 0;
-#pragma unroll(LAG || !std::is_same<VP2, VehP2>::value ? kSpecUnroll : 1)
+#pragma unroll(LAG || !std::is_same<VP2, VehP2>::value ? kTickUnroll : 1)
         for (int j = 0; j < n; ++j) inner_tick_pair_spec<LAG>(d, u, v2, rare);
         flown = !__any_sync(__activemask(), rare != 0);
-#if UAVB_SPEC_COUNT
-        const unsigned am = __activemask();
-        const bool lim = __any_sync(am, (rare >> kRareLimitBit) & 1u), rot = __any_sync(am, (rare >> kRareRotBit) & 1u);
-        if ((threadIdx.x & 31u) == (unsigned)(__ffs(am) - 1)) {
-          atomicAdd(&g_spec_count[2], 1ull);
-          if (!flown) atomicAdd(&g_spec_count[3], 1ull);
-          if (lim) atomicAdd(&g_spec_count[4], 1ull);
-          if (rot) atomicAdd(&g_spec_count[5], 1ull);
-        }
-#endif
         if (!flown) {                                        // roll back: the same n ticks with the exact body
           slot.load(d);
           hold = kSpecHold + 1;
         }
       }
       if (!watch && hold > 0) --hold;
-#if UAVB_SPEC_COUNT
-      if ((threadIdx.x & 31u) == (unsigned)(__ffs(__activemask()) - 1)) atomicAdd(&g_spec_count[watch ? 0 : 1], 1ull);
-#endif
       if (watch) {
         stretch(BoolC<true>{});
       } else if (!flown) {

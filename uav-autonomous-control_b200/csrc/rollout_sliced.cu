@@ -6,6 +6,4 @@ namespace uavb {
 UAVB_LAUNCH_PAIR(kTargetFly, 0);
 UAVB_LAUNCH_PAIR(kTargetShared, 0);
 
-cudaError_t spec_counts_sliced(unsigned long long* counts, bool reset) { return spec_counts<0>(counts, reset); }
-
 }  // namespace uavb

@@ -7,6 +7,4 @@ namespace uavb {
 UAVB_LAUNCH_PAIR(kTargetPerRollout, 0);
 UAVB_LAUNCH_PAIR(kTargetPerRollout, 3);
 
-cudaError_t spec_counts_tables(unsigned long long* counts, bool reset) { return spec_counts<0>(counts, reset); }
-
 }  // namespace uavb
