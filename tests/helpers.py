@@ -62,3 +62,21 @@ def mc_arrays(dev, B, gain_scale=None, mass_scale=None, inertia_scale=None, wind
     if wind is not None:
         out["mc_wind"] = torch.tensor(np.asarray(wind, float).reshape(B, 3).T.copy(), dtype=torch.float32, device=dev).contiguous()
     return out
+
+
+def hover_table(start):
+    """A one-row trajectory table: hold a point 0.2 m / -0.1 m off the start at 1 m altitude, yaw 0.4 rad."""
+    return np.array([[start[0] + 0.2, start[1] - 0.1, -1.0, 0, 0, 0, 0, 0, 0, 0.4, 0]])
+
+
+def rough_mc(dev, B, seed=11, tumble=False):
+    """Wind +-0.3 N and gains x U(0.5, 1.5) (most stretches of a warp see some lane at a rotor limit); tumble: every other rollout is a
+    low-inertia vehicle with four times the attitude gains (with a yaw set-point 3 rad away, |w| goes well above 44.7 rad/s)."""
+    rng = np.random.default_rng(seed)
+    gains = rng.uniform(0.5, 1.5, (B, 11))
+    inertia = np.ones((B, 3))
+    if tumble:
+        gains[::2] = 1.0
+        gains[::2, [5, 6, 8, 9]] = 4.0
+        inertia[::2] = 0.1
+    return mc_arrays(dev, B, gain_scale=gains, inertia_scale=inertia, wind=rng.uniform(-0.3, 0.3, (B, 3)))

@@ -10,7 +10,7 @@ import ctypes
 import numpy as np
 import pytest
 
-from helpers import lab_course_plan, mc_arrays
+from helpers import hover_table, lab_course_plan, mc_arrays, rough_mc
 
 START = np.array([1.0, 7.0, -0.021])            # lab_course start
 FREQ = 10
@@ -65,7 +65,7 @@ def _both(spec, plan, B, n_ticks, dev, **kw):
 
 
 def _hover_table():
-    return np.array([[START[0] + 0.2, START[1] - 0.1, -1.0, 0, 0, 0, 0, 0, 0, 0.4, 0]])
+    return hover_table(START)
 
 
 def _bench_setup(dev, B):
@@ -79,17 +79,7 @@ def _bench_setup(dev, B):
     return plan, 10 * int(plan.total_rows.sum()), kw, torch
 
 
-def _rough(dev, B, seed=11, tumble=False):
-    """Wind +-0.3 N and gains x U(0.5, 1.5) (most stretches of a warp see some lane at a rotor limit); tumble: every other rollout is a
-    low-inertia vehicle with four times the attitude gains and a yaw set-point 3 rad away (|w| well above 44.7 rad/s, C oracle)."""
-    rng = np.random.default_rng(seed)
-    gains = rng.uniform(0.5, 1.5, (B, 11))
-    inertia = np.ones((B, 3))
-    if tumble:
-        gains[::2] = 1.0
-        gains[::2, [5, 6, 8, 9]] = 4.0
-        inertia[::2] = 0.1
-    return mc_arrays(dev, B, gain_scale=gains, inertia_scale=inertia, wind=rng.uniform(-0.3, 0.3, (B, 3)))
+_rough = rough_mc
 
 
 @pytest.mark.gpu

@@ -159,6 +159,11 @@ enum : int { kTargetFly = 0, kTargetShared = 1, kTargetPerRollout = 2 };
 // Non-watching stretches flown with the exact body after a rollback (rare paths cluster in mission phases): 4 against 0 / 16 gives
 // 4.40 against 4.64 / 4.41 ms (profiles/r03_spec_probe.jsonl).
 constexpr int kSpecHold = 4;
+
+// The tan-form quaternion map of the pair tick grows |q| by 1/cos(dt |w| / 2) per tick on purpose, and renormalise_q_pair's
+// 1.5 - 0.5 |q|^2 is exact to O(e^2) only: the metrics-only bodies renormalise at every phase that is a multiple of kNormTicks as well as
+// at the end of each outer period, so that periods longer than 10 ticks (frequency > 10) let the norm grow no further than at 10.
+constexpr int kNormTicks = 10;
 constexpr int kSpecSlotVec4 = 10;                            // 20 float2 fields of Drone2 = 10 x 16 bytes per thread
 template <int MODE, class LOG> constexpr bool kSpecBody = std::is_same<LOG, NoPairLog>::value && MODE != kTargetFly;
 
@@ -314,6 +319,12 @@ UAVB_DEV void rollout_run_pair(Drone2& d, Cursor<float> (&c)[2], Accum<float> (&
   constexpr bool kSpec = kSpecBody<MODE, LOG>;
   int hold = 0;                                              // non-watching stretches left to fly exactly (not carried: no effect on results)
   if constexpr (kSpec) hold = slot.exact ? 0x7fffffff : 0;
+  // periods longer than kNormTicks split their stretches (below); a separate copy of the loop, so that shorter periods fly the same
+  // code as without the split, and one tick per iteration there (unrolled, the second copy of the body spills at 255 registers).
+  // kTargetFly bodies (fp64 set-points evaluated inline) keep one loop that splits at run time: a second copy spills there.
+  const bool long_period = !LOG::kNormEveryTick && freq > kNormTicks;   // (launch-uniform)
+  auto run = [&](auto long_c) {
+  constexpr bool kLong = decltype(long_c)::value;
   while (k < n_ticks) {
     if (c[0].phase == 0) {
       Target2<typename PairTarget<MODE>::T> t;
@@ -322,7 +333,12 @@ UAVB_DEV void rollout_run_pair(Drone2& d, Cursor<float> (&c)[2], Accum<float> (&
       c[0].ex = ex.x; c[1].ex = ex.y; c[0].ey = ey.x; c[1].ey = ey.y; c[0].ez = ez.x; c[1].ez = ez.y;
       outer_update_pair(d, u, vo, t, ex, ey, ez);
     }
-    const int n = (freq - c[0].phase < n_ticks - k) ? (freq - c[0].phase) : (n_ticks - k);
+    // stretches also end where the phase reaches a multiple of kNormTicks (below): F <= kNormTicks keeps one stretch per period
+    int n = (freq - c[0].phase < n_ticks - k) ? (freq - c[0].phase) : (n_ticks - k);
+    if (kLong && long_period) {
+      const int to_norm = kNormTicks - c[0].phase % kNormTicks;
+      n = to_norm < n ? to_norm : n;
+    }
     bool watch = false;
     if (OBST::kAny) watch = __any_sync(__activemask(), pair_watch(d, a, u, acc_max, oa, ob, n, clear, gr));   // one decision per warp; watching is always correct
     auto stretch = [&](auto watch_c) {
@@ -333,7 +349,7 @@ UAVB_DEV void rollout_run_pair(Drone2& d, Cursor<float> (&c)[2], Accum<float> (&
       // waits for instruction fetches and runs 10 % slower (measured).  Per-rollout tables unroll only without a state log: with
       // Monte-Carlo overrides and per-thread log stores the unrolled body no longer fits 255 registers (ptxas spills), and a
       // logging launch is bound by its HBM stores anyway.
-#pragma unroll((kWatch || MODE == kTargetFly || (MODE == kTargetPerRollout && LOG::kNormEveryTick)) ? 1 : kTickUnroll)
+#pragma unroll((kLong || kWatch || MODE == kTargetFly || (MODE == kTargetPerRollout && LOG::kNormEveryTick)) ? 1 : kTickUnroll)
       for (int j = 0; j < n; ++j) {
         inner_tick_pair<LOG::kNormEveryTick, LAG>(d, u, v2);
         if constexpr (kWatch) {
@@ -349,7 +365,7 @@ UAVB_DEV void rollout_run_pair(Drone2& d, Cursor<float> (&c)[2], Accum<float> (&
       if (!watch && hold == 0) {                             // (warp-uniform)
         slot.save(d);
         unsigned rare = 0;
-#pragma unroll(LAG || !std::is_same<VP2, VehP2>::value ? kTickUnroll : 1)
+#pragma unroll(!kLong && (LAG || !std::is_same<VP2, VehP2>::value) ? kTickUnroll : 1)
         for (int j = 0; j < n; ++j) inner_tick_pair_spec<LAG>(d, u, v2, rare);
         flown = !__any_sync(__activemask(), rare != 0);
         if (!flown) {                                        // roll back: the same n ticks with the exact body
@@ -387,8 +403,16 @@ UAVB_DEV void rollout_run_pair(Drone2& d, Cursor<float> (&c)[2], Accum<float> (&
       d.px[0] += (double)d.dx.x; d.py[0] += (double)d.dy.x; d.pz[0] += (double)d.dz.x;
       d.px[1] += (double)d.dx.y; d.py[1] += (double)d.dy.y; d.pz[1] += (double)d.dz.y;
       d.dx = d.dy = d.dz = make_float2(0.f, 0.f);
+    } else if (kLong && long_period && c[0].phase % kNormTicks == 0) {
+      renormalise_q_pair(d);   // within a long period too, on the phase (not where a launch ends)
     }
     c[1].phase = c[0].phase;
+  }
+  };
+  if constexpr (MODE == kTargetFly) {
+    run(BoolC<!LOG::kNormEveryTick>{});
+  } else {
+    if (long_period) run(BoolC<true>{}); else run(BoolC<false>{});
   }
 #pragma unroll
   for (int l = 0; l < 2; ++l) {

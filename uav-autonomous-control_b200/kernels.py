@@ -617,13 +617,20 @@ def rollout(plan, B: int, n_ticks: int, *, start: torch.Tensor, goal: Optional[t
     flown-path list (MujocoSimulation._record_actual_trajectory, mujoco_sim.py:201-218): positions every traj_interval seconds
     of simulation time while z <= traj_gate_z, into result.traj [traj_max_samples, 3, B] / result.traj_count [B].
     ``plan``: a MissionPlan (waypoint missions), or a TablePlan (``plan_tables``: caller trajectory tables, one row per
-    ``frequency`` ticks; fp32 only).
+    ``frequency`` ticks; fp32 only).  A MissionPlan's table period ``plan.dt`` must equal ``vehicle.dt * frequency`` (to 1e-12
+    relative): it is also the outer-loop dt of the controller (altitude integral, set-point times), which the reference takes as
+    ``quad.dt * frequency`` for both (main.py:97); a mismatch raises ValueError.  A TablePlan takes its outer dt from
+    ``vehicle.dt * frequency``.
     """
     tables = isinstance(plan, TablePlan)
     dev = plan.rows.device if tables else plan.seg_coeffs.device
     f64 = dtype == torch.float64
     if tables and f64:
         raise ValueError("trajectory tables fly in the fp32 rollout only (uavb_rollout_f64 takes waypoint missions)")
+    veh = vehicle if vehicle is not None else nat.default_vehicle()
+    if not tables and frequency >= 1 and abs(plan.dt - veh.dt * frequency) > 1e-12 * abs(veh.dt * frequency):
+        raise ValueError(f"the plan is sampled at dt = {plan.dt}, but vehicle.dt * frequency = {veh.dt} * {frequency} = {veh.dt * frequency}: "
+                         "plan the mission at vehicle.dt * frequency")
     odt = torch.float64 if f64 else torch.float32
     a = nat.RolloutArgs()
     a.B, a.n_ticks, a.inner_per_outer = int(B), int(n_ticks), int(frequency)
@@ -634,7 +641,7 @@ def rollout(plan, B: int, n_ticks: int, *, start: torch.Tensor, goal: Optional[t
     a.pair_kernel_only = int(bool(pair_kernel_only))
     if ground_z is not None:
         a.ground_on, a.ground_z = 1, float(ground_z)
-    a.veh = vehicle if vehicle is not None else nat.default_vehicle()
+    a.veh = veh
     a.mc_mass = nat.ptr(mc_mass, torch.float32, "mc_mass")
     a.mc_inertia = nat.ptr(mc_inertia, torch.float32, "mc_inertia")
     a.mc_gains = nat.ptr(mc_gains, torch.float32, "mc_gains")
